@@ -46,6 +46,28 @@ def kernel_constants():
 
 
 # ----------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed paths return to their caller, for comparing two builds output for output
+# ----------------------------------------------------------------------------------------------
+DUMP_MAX_BYTES = 64 << 20
+DUMP_COMPARE_CELLS = 1 << 20   # at most this many of the parity check's seeded sample of matrix cells
+
+
+def hash_words(h):
+    """uint64 hashes as an (n, 2) float64 array of their high and low 32-bit halves: exact, where one float64 per
+    hash would round every hash above 2**53"""
+    return np.stack([(h >> np.uint64(32)).astype(np.float64), (h & np.uint64(0xFFFFFFFF)).astype(np.float64)], axis=1)
+
+
+def dump_outputs(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "outputs to dump are %d bytes, more than %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+# ----------------------------------------------------------------------------------------------
 # synthetic inputs
 # ----------------------------------------------------------------------------------------------
 def np_genome(n, seed):
@@ -221,7 +243,7 @@ def run_reference(args):
     if not args.no_compare:
         nb = min(args.compare_sketches, 2000)
         rows = planted_sketches(nb, 500, 0x5EED0100)
-        c_steps = max(1, min(args.steps, 3))
+        c_steps = args.steps
         cpu_compare_rate(rows[:256], threads)
         t0 = time.perf_counter()
         for _ in range(c_steps):
@@ -419,6 +441,11 @@ def run_ours(args):
     smb.profile_enable(False)
     value = total_bases / (ms_dev * 1e-3) / 1e9
     md5_dev = [m.md5sum() for m in mhs]
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    if outputs is not None:   # the three sketches after the last timed step, as kmerminhash_get_mins / _get_abunds give them
+        for k, m in zip(KSIZES, mhs):
+            outputs["sketch_k%d_mins" % k] = hash_words(m.mins_np())
+            outputs["sketch_k%d_abunds" % k] = m.abunds_np().astype(np.float64)
 
     # ---- end-to-end path: pinned host buffers in, sketches read back every step ------------------------
     ms_e2e, d2h_total, mhs2 = timed_e2e(KSIZES)
@@ -502,7 +529,7 @@ def run_ours(args):
         T = max(1, min(args.percall_threads or 4, host_threads))
         z = np.zeros((R, READ_LEN + 1), dtype=np.uint8)
         z[:, :READ_LEN] = host_batches[0].numpy().reshape(R, READ_LEN)
-        pc_steps = max(1, min(args.steps, 3))
+        pc_steps = args.steps
         warm_reads = min(R // T // 8, 50_000)
         secs, groups = 0.0, None
         barrier()
@@ -552,7 +579,7 @@ def run_ours(args):
     compare = None
     if not args.no_compare:
         compare = bench_compare(args, smb, torch, dist, dev, rank, world, barrier, max_over_ranks, lib_stream, windows,
-                                host_threads, hbm_peak, peak_src)
+                                host_threads, hbm_peak, peak_src, outputs)
 
     clocks.stop()
 
@@ -643,13 +670,15 @@ def run_ours(args):
             "clocks": clk,
             "compare": compare,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
 
 
 def bench_compare(args, smb, torch, dist, dev, rank, world, barrier, max_over_ranks, lib_stream, windows, host_threads,
-                  hbm_peak, peak_src):
+                  hbm_peak, peak_src, outputs):
     N, NUM = args.compare_sketches, 500
     rows = planted_sketches(N, NUM, 0x5EED0100)
     from sourmash_rust_b200 import sharding
@@ -664,7 +693,7 @@ def bench_compare(args, smb, torch, dist, dev, rank, world, barrier, max_over_ra
     common = torch.empty((max(1, nr), N), dtype=torch.int32, device=dev)
     size = torch.empty((max(1, nr), N), dtype=torch.int32, device=dev)
     ratio = torch.empty((max(1, nr), N), dtype=torch.float64, device=dev)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
 
     def step():
         # all-gather of the packed sketches over NCCL/NVLink + this rank's row block, in one library call: the
@@ -706,17 +735,22 @@ def bench_compare(args, smb, torch, dist, dev, rank, world, barrier, max_over_ra
               np.array_equal(gr, oc.astype(np.float64) / np.maximum(1, osz).astype(np.float64)))
     assert ok, "rank %d: sampled pairs differ from the oracle" % rank
     nonzero = int((oc > 0).sum())
+    if outputs is not None:   # the last timed step's matrix at (a prefix of) the seeded sample of cells just checked
+        m = min(n_s, DUMP_COMPARE_CELLS)
+        outputs.update(compare_rows=(r0 + ii[:m]).astype(np.float64), compare_cols=jj[:m].astype(np.float64),
+                       compare_common=gc[:m].astype(np.float32), compare_size=gs[:m].astype(np.float32),
+                       compare_ratio=gr[:m].astype(np.float64))
 
     # ---- the same matrix with the data-driven path choice overridden: every pair walked (dense kernel) --------------------
     smb.compare_path("dense")
     step()
     barrier()
     e0.record(lib_stream)
-    for _ in range(2):
+    for _ in range(steps):
         step()
     e1.record(lib_stream)
     barrier()
-    ms_dense = max_over_ranks(e0.elapsed_time(e1)) / 2
+    ms_dense = max_over_ranks(e0.elapsed_time(e1)) / steps
     smb.compare_path("auto")
 
     # ---- end to end: host CSR in, f64 Jaccard matrix out to pinned host memory ----------------------------------------------
@@ -792,7 +826,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-percall", action="store_true")
     ap.add_argument("--no-packed", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write, as DIR/<name>.npy (float32/float64), what the timed paths computed in "
+                         "their last step: the three sketches' hashes (high and low 32 bits) and abundances, and the "
+                         "compare matrix at a seeded sample of cells")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
