@@ -572,8 +572,10 @@ std::vector<std::vector<uint64_t>> linear_find_lists(SketchCollection &index, Sk
         for (uint32_t v : index.h_nums) index_unbounded &= v == 0;
         const bool count_sim = mode == 0 && index_unbounded;
         const bool count_path = (mode == 1 || count_sim) && threshold >= 0.0;
-        // a large index against a (much) smaller query batch: stream the index at HBM rate (find_stream.cu)
-        const bool stream = count_path && g_find_path != 1 && queries.n_hashes > 0 && queries.n_hashes < (1ull << 31) && nq < (1ull << 31) &&
+        // a large index against a (much) smaller query batch: stream the index at HBM rate (find_stream.cu); the query
+        // table's slot numbers (twice the query hashes + 32 per table slice) are u32
+        const bool stream = count_path && g_find_path != 1 && queries.n_hashes > 0 && queries.n_hashes < (1ull << 31) &&
+                            find_stream_table_slots(queries.n_hashes) <= (1ull << 32) && nq < (1ull << 31) &&
                             index.max_len < (1u << 31) &&
                             (g_find_path >= 2 || (index.n_hashes >= 4 * queries.n_hashes && index.n_hashes >= (1ull << 22)));
         uint32_t *q_tstart = nullptr;

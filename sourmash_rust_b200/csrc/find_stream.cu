@@ -158,8 +158,11 @@ __global__ void __launch_bounds__(128) qt_sums_kernel(const uint32_t *__restrict
     __syncthreads();
     if (threadIdx.x == 0) sums[t] = part[0] + part[1] + part[2] + part[3];
 }
-// tstart[t] = first slot of slice t: every slice gets twice its postings + 32 slots
-__global__ void __launch_bounds__(1024) qt_starts_kernel(const unsigned long long *__restrict__ sums, uint32_t *tstart) {
+// tstart[t] = first slot of slice t: every slice gets twice its postings + 32 slots.  Also empties the slot of its own
+// at tstart[QT_SLICES] that holds the list of the one hash that looks like an empty slot (~0): it must be empty before
+// ANY CTA of qtable_slice_kernel runs, since the last slice's CTA pushes onto it while the others still start up.
+__global__ void __launch_bounds__(1024) qt_starts_kernel(const unsigned long long *__restrict__ sums, uint32_t *tstart,
+                                                         unsigned long long *tkey, int32_t *thead) {
     __shared__ uint32_t sz[QT_SLICES];
     const uint32_t t = threadIdx.x;
     sz[t] = (uint32_t)(2 * (sums[t + 1] - sums[t]) + 32);
@@ -168,6 +171,8 @@ __global__ void __launch_bounds__(1024) qt_starts_kernel(const unsigned long lon
         uint32_t acc = 0;
         for (uint32_t i = 0; i < QT_SLICES; i++) { tstart[i] = acc; acc += sz[i]; }
         tstart[QT_SLICES] = acc;
+        tkey[acc] = FS_EMPTY;
+        thead[acc] = -1;
     }
 }
 template <bool SHARED>
@@ -193,10 +198,6 @@ __global__ void __launch_bounds__(1024) qtable_slice_kernel(const uint64_t *__re
     unsigned long long *key = in_smem ? s_key : tkey + start;
     int32_t *head = in_smem ? reinterpret_cast<int32_t *>(s_key + QT_SMEM_SLOTS) : thead + start;
     for (uint32_t i = threadIdx.x; i < size; i += blockDim.x) { key[i] = FS_EMPTY; head[i] = -1; }
-    if (t == 0 && threadIdx.x == 0) {   // the slot of its own of the one hash that looks like an empty slot
-        tkey[tstart[QT_SLICES]] = FS_EMPTY;
-        thead[tstart[QT_SLICES]] = -1;
-    }
     __syncthreads();
     // a thread takes a query at a time: the (few) postings of that query inside this slice
     for (uint64_t q = threadIdx.x; q < nq; q += blockDim.x) {
@@ -472,7 +473,7 @@ void launch_qtable_build(const uint64_t *qh, const uint64_t *qo, uint64_t nq, ui
     launch_part_offsets(qh, qo, nq, tscale, QT_SLICES, qpo, st);
     qt_sums_kernel<<<QT_SLICES + 1, 128, 0, st>>>(qpo, nq, sums);
     SM_LAUNCHED();
-    qt_starts_kernel<<<1, QT_SLICES, 0, st>>>(sums, tstart);
+    qt_starts_kernel<<<1, QT_SLICES, 0, st>>>(sums, tstart, tkey, thead);
     SM_LAUNCHED();
     static bool attr_set = false;
     const size_t smem = (size_t)QT_SMEM_SLOTS * 12;
