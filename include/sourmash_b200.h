@@ -152,21 +152,9 @@ uint64_t smgpu_scaffold_pairs(SketchCollection *c, uint64_t *pairs_first, uint64
  * only those are walked when the (pair, shared hash) incidences are few against the dense work;
  * 1 forces the dense tile kernel, 2 forces the inverted-index path, 3 = as 0 but with the
  * sorted-postings join instead of the hash-grouped one (the default; it builds a hash table over
- * the ROW block's hashes only, so a row shard of an all-vs-all matrix costs its share of the rows),
- * 4 = as 2, and a block whose probe found many incidences is not handed to the dense kernels.
- * Results are identical. */
+ * the ROW block's hashes only, so a row shard of an all-vs-all matrix costs its share of the rows).
+ * Any other value selects 0.  Results are identical. */
 void smgpu_compare_path(int32_t path);
-/* How the related pairs of a block are walked (src/lib.rs:470-499 per pair): 0 (default) = one thread per pair;
- * 2 = one warp per pair (merge-path split over the lanes, both lists staged in shared memory) where the two
- * sketches together hold at most 1024 hashes.  Results are identical; the warp form measured slower and is kept for
- * A/B runs (DESIGN.md section 8). */
-void smgpu_walk_form(int32_t form);
-/* smgpu_compare_matrix_allgather with device outputs over sketches of one length (full `num` sketches): with
- * `stages` > 1 the gathered hashes travel in that many groups of point-to-point exchanges (peers by ring distance) and
- * the join probes each group's sketches while the next group is on the wire.  1 (default; SMB200_GATHER_STAGES) = one
- * ncclAllGather, the join's probe behind it -- measured equal or faster on 4 GPUs (DESIGN.md section 8).  Returns the previous value; `stages` < 1 only reads it.  Every rank must use the same value.
- * Results are identical. */
-int32_t smgpu_gather_stages(int32_t stages);
 /* How smgpu_linear_find counts shared hashes when a count decides the hit (containment; similarity of sketches
  * without a num): 0 (default) = an index that is large against the query batch is STREAMED once past per-slice
  * Bloom filters of the query hashes held in shared memory (the search then runs at the rate HBM delivers the

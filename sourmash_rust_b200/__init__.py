@@ -109,8 +109,6 @@ EXTENSION_ABI = {
     "smgpu_scaffold_pairs": (u64, [vp, vp, vp]),
     "smgpu_compare_path": (None, [i32]),
     "smgpu_find_path": (None, [i32]),
-    "smgpu_walk_form": (None, [i32]),
-    "smgpu_gather_stages": (i32, [i32]),
     "smgpu_linear_find": (u64, [vp, vp, i32, C.c_double, vp, vp, u64]),
     "smgpu_comm_unique_id": (None, [vp]),
     "smgpu_comm_init": (None, [vp, i32, i32]),
@@ -220,17 +218,7 @@ PROFILE_KINDS = {"sketch_k21": 0, "sketch_k31": 1, "sketch_k51": 2, "sketch_othe
 
 def compare_path(path="auto"):
     """'auto' | 'dense' | 'sparse' | 'noprobe' (smgpu_compare_path)"""
-    lib().smgpu_compare_path({"auto": 0, "dense": 1, "sparse": 2, "noprobe": 3, "probe": 4}[path])
-
-
-def gather_stages(stages=0):
-    """groups of the staged gather in compare_matrix_allgather (smgpu_gather_stages); returns the previous value"""
-    return lib().smgpu_gather_stages(int(stages))
-
-
-def walk_form(form="thread"):
-    """'thread' | 'warp' (smgpu_walk_form)"""
-    lib().smgpu_walk_form({"thread": 0, "warp": 2}[form])
+    lib().smgpu_compare_path({"auto": 0, "dense": 1, "sparse": 2, "noprobe": 3}[path])
 
 
 def find_path(path="auto"):

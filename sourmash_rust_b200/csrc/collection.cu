@@ -146,14 +146,14 @@ int g_find_path = [] {
     const char *e = getenv("SMB200_FIND_PATH");
     return e ? atoi(e) : 0;
 }();
-// How the related pairs are walked: 0 (default) = one thread per pair; 2 = one WARP per pair (merge-path split, lists
-// in shared memory) where both sketches together hold at most 1024 hashes.  The warp form is exact and kept for A/B
-// runs -- it measured 3.8x SLOWER than the thread form on cfg3 (DESIGN.md section 8).  SMB200_WALK_FORM / smgpu_walk_form.
-int g_walk_form = [] {
-    const char *e = getenv("SMB200_WALK_FORM");
-    return e ? atoi(e) : 0;
-}();
 int g_compare_path = 0;  // 0 = choose from the data, 1 = dense tile kernel, 2 = inverted-index path, 3 = inverted index without the probe form
+
+// The part of the probe-form decision that the compare path and the row collection make: forced sparse always probes;
+// by default a block probes unless an earlier probe over the same rows found the dense kernels the better choice.
+// The block's size tests come on top (compare_block_device; compare_matrix_allgather decides before the gather).
+bool probe_form_allowed(const SketchCollection &rows) {
+    return (g_compare_path == 0 && !rows.probe_dense_preferred) || g_compare_path == 2;
+}
 
 static int bit_length64(uint64_t x) {
     int b = 0;
@@ -217,15 +217,9 @@ void join_table_build(Context &ctx, JoinTable &jt, const uint64_t *bh, const uin
 // One block of the matrix into DEVICE outputs.  Picks the sparse path (inverted index: only pairs
 // sharing a hash are walked) when the number of (pair, shared hash) incidences is small against
 // the dense work, else the dense tile kernel.  Same integers either way.
-void wait_arrivals(cudaStream_t st, const std::vector<ColumnArrival> *arrivals) {
-    if (!arrivals) return;
-    for (const ColumnArrival &a : *arrivals)
-        if (a.ready) SM_CUDA(cudaStreamWaitEvent(st, a.ready, 0));
-}
-
 void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, SketchCollection &cols, uint64_t c0,
                           uint64_t nc, int mode, uint32_t *common, uint32_t *size, double *ratio, uint64_t ld,
-                          const JoinTable *prebuilt, const std::vector<ColumnArrival> *arrivals) {
+                          const JoinTable *prebuilt, cudaEvent_t cols_ready) {
     Context &ctx = Context::get();
     cudaStream_t st = ctx.stream;
     const uint64_t *rh = rows.d_hashes.as<uint64_t>(), *ro = rows.d_offsets.as<uint64_t>();
@@ -237,7 +231,7 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
     const uint64_t n_r = shared ? 0 : rows.h_offsets[r0 + nr] - rows.h_offsets[r0];
     const uint64_t n_c = cols.h_offsets[c0 + nc] - cols.h_offsets[c0];
     const uint64_t n = n_r + n_c;
-    const bool force_dense = g_compare_path == 1, force_sparse = g_compare_path == 2 || g_compare_path == 4;
+    const bool force_dense = g_compare_path == 1, force_sparse = g_compare_path == 2;
     const bool big = n > 0 && nr * nc >= 4096 && nr < (1ull << 31) && nc < (1ull << 31);
     bool sparse = !force_dense && n > 0 && (force_sparse || big) && nr < (1ull << 31) && nc < (1ull << 31);
     // full num sketches (Jaccard): the dense walk can run on 32-bit ranks with a fixed trip count
@@ -262,29 +256,12 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
     const uint64_t n_bp = build_cols ? n_c : n_rp, n_build = build_cols ? nc : nr;
     const uint64_t *bh = build_cols ? ch : rh, *bo = build_cols ? co : ro, *ph = build_cols ? rh : ch, *po = build_cols ? ro : co;
     const uint64_t b0 = build_cols ? c0 : r0, p0 = build_cols ? r0 : c0, n_probe = build_cols ? nr : nc;
-    const bool probe = sparse && g_compare_path != 3 && n_bp > 0 && n_bp < (1ull << 31) &&
-                       !(rows.probe_dense_preferred && !force_sparse);
-    // Column hashes still in flight: the probe form with the table over the ROWS takes the parts as they land (each part
-    // is its own probe launch, behind that part's event); everything else needs all of them now.
-    const bool staged = arrivals && probe && !build_cols && c0 == 0;
-    if (arrivals && !staged) wait_arrivals(st, arrivals);
-    auto probe_columns = [&](bool count, const unsigned long long *tkey, const uint64_t *toff, const uint32_t *grows, int log2_t,
-                             uint32_t *cmat, uint64_t cld, unsigned long long *bitmap, const uint32_t *filter, int log2_f) {
-        if (!staged) {
-            launch_probe_group(count, build_cols, tkey, toff, grows, log2_t, ph, po, p0, n_probe, cmat, cld, bitmap, n_build, ctx.dsc(SC_CNT),
-                               filter, log2_f, st);
-            return;
-        }
-        uint64_t covered = 0;
-        for (const ColumnArrival &a : *arrivals) {
-            if (a.c_end > nc || a.c_begin > a.c_end) throw_internal("column arrivals outside the block");
-            if (a.ready) SM_CUDA(cudaStreamWaitEvent(st, a.ready, 0));
-            launch_probe_group(count, false, tkey, toff, grows, log2_t, ph, po, p0, a.c_end - a.c_begin, cmat, cld, bitmap, n_build,
-                               ctx.dsc(SC_CNT), filter, log2_f, st, a.c_begin);
-            covered += a.c_end - a.c_begin;
-        }
-        if (covered != nc) throw_internal("column arrivals do not cover the block");
-    };
+    const bool probe = sparse && n_bp > 0 && n_bp < (1ull << 31) && probe_form_allowed(rows);
+    // Column hashes still in flight: the probe form with the table over the ROWS waits for them right before its probe
+    // launch (what it queues first needs the rows and the column offsets only); everything else needs them now.
+    cudaEvent_t probe_waits = nullptr;
+    if (probe && !build_cols) probe_waits = cols_ready;
+    else if (cols_ready) SM_CUDA(cudaStreamWaitEvent(st, cols_ready, 0));
     if (probe) {
         // the table: handed in (built over exactly this block's build side, on this thread's scratch) or built here;
         // with a presence filter in front of it when the probing side is a different, larger collection
@@ -314,7 +291,9 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
                 cld = nc;
             }
             SM_CUDA(cudaMemset2DAsync(cmat, cld * 4, 0, nc * 4, nr, st));
-            probe_columns(true, tkey, toff, grows, log2_t, cmat, cld, nullptr, filter, log2_f);
+            if (probe_waits) SM_CUDA(cudaStreamWaitEvent(st, probe_waits, 0));
+            launch_probe_group(true, build_cols, tkey, toff, grows, log2_t, ph, po, p0, n_probe, cmat, cld, nullptr, n_build,
+                               ctx.dsc(SC_CNT), filter, log2_f, st);
             if (size || ratio || cmat != common)  // (counts only, straight into the caller's matrix: nothing left to do)
                 launch_fill_cells(ro, rnum, r0, nr, co, c0, nc, 1, cmat, cld, common, size, ratio, ld, st);
         } else {
@@ -326,7 +305,9 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
             SM_CUDA(cudaMemsetAsync(bitmap, 0, n_words * 8, st));
             // (the unrelated-pair values need row lengths only: written first, they overlap a transfer the probe waits for)
             launch_fill_cells(ro, rnum, r0, nr, co, c0, nc, 0, nullptr, 0, common, size, ratio, ld, st);  // as if unrelated
-            probe_columns(false, tkey, toff, grows, log2_t, nullptr, 0, bitmap, filter, log2_f);
+            if (probe_waits) SM_CUDA(cudaStreamWaitEvent(st, probe_waits, 0));
+            launch_probe_group(false, build_cols, tkey, toff, grows, log2_t, ph, po, p0, n_probe, nullptr, 0, bitmap, n_build,
+                               ctx.dsc(SC_CNT), filter, log2_f, st);
             launch_popc_words(bitmap, n_words, counts, st);
             scan_exclusive_u64(counts, pre, n_words, ctx.scan_tmp.p, st);
             // the pair list can hold every cell of a block of up to 2^26 cells: then the walk reads its
@@ -342,13 +323,8 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
                 launch_expand_bits(bitmap, pre, n_words, ctx.join[5].as<uint64_t>(), st, cap);
                 // the whole square of ONE collection whose sketches share a `num`: each unordered pair is walked once
                 const bool symmetric = (&rows == &cols) && r0 == c0 && nr == nc && rows.uniform_num(r0, nr);
-                // short sketches (both together at most 1024 hashes): one warp per pair, lists in shared memory (join.cu)
-                if (g_walk_form == 2 && walk_pairs_warp_fits(rows.max_len, cols.max_len))
-                    launch_walk_pairs_warp(ctx.join[5].as<uint64_t>(), cap, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st,
-                                           pre + (n_words - 1), counts + (n_words - 1), build_cols ? 0 : nr, symmetric);
-                else
-                    launch_walk_pairs(ctx.join[5].as<uint64_t>(), cap, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st,
-                                      pre + (n_words - 1), counts + (n_words - 1), build_cols ? 0 : nr, symmetric);  // probe-major cell ids
+                launch_walk_pairs(ctx.join[5].as<uint64_t>(), cap, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st,
+                                  pre + (n_words - 1), counts + (n_words - 1), build_cols ? 0 : nr, symmetric);  // probe-major cell ids
             }
         }
         // The probe path is exact whatever the data; whether the dense kernels would have been faster
@@ -436,10 +412,7 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
     if (n_pairs) {
         ctx.join[5].reserve((n_pairs + 1) * 8);
         launch_expand_bits(bitmap, pre, n_words, ctx.join[5].as<uint64_t>(), st);
-        if (g_walk_form == 2 && walk_pairs_warp_fits(rows.max_len, cols.max_len))
-            launch_walk_pairs_warp(ctx.join[5].as<uint64_t>(), n_pairs, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st);
-        else
-            launch_walk_pairs(ctx.join[5].as<uint64_t>(), n_pairs, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st);
+        launch_walk_pairs(ctx.join[5].as<uint64_t>(), n_pairs, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st);
     }
 }
 

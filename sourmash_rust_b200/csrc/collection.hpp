@@ -60,23 +60,17 @@ struct JoinTable {
 };
 void join_table_build(Context &ctx, JoinTable &jt, const uint64_t *bh, const uint64_t *bo, uint64_t b0, uint64_t n_build,
                       uint64_t n_bp, bool with_filter, cudaStream_t side = nullptr, cudaEvent_t side_go = nullptr);
-// Columns [c_begin, c_end) of a block (block-local ids) are in device memory once `ready` has passed on the stream that
-// waits for it (null: they already are).  A gathered collection whose parts are still in flight is described by a list of
-// these covering all its columns (comm.cu); offsets and nums of ALL columns are valid from the start.
-struct ColumnArrival {
-    uint64_t c_begin = 0, c_end = 0;
-    cudaEvent_t ready = nullptr;
-};
-void wait_arrivals(cudaStream_t st, const std::vector<ColumnArrival> *arrivals);
-// one block of the matrix into device outputs (common / size / ratio may be null).  `arrivals` (optional): the column
-// hashes arrive in parts; the probe form of the join then probes each part as it lands, every other form waits for all.
+// one block of the matrix into device outputs (common / size / ratio may be null).  `cols_ready` (optional): the column
+// hashes are in device memory once this event has passed on the calling thread's stream (null: they already are); their
+// offsets and nums are valid from the start (a gathered collection still in flight, comm.cu).
 void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, SketchCollection &cols, uint64_t c0, uint64_t nc,
                           int mode, uint32_t *common, uint32_t *size, double *ratio, uint64_t ld,
-                          const JoinTable *prebuilt = nullptr, const std::vector<ColumnArrival> *arrivals = nullptr);
+                          const JoinTable *prebuilt = nullptr, cudaEvent_t cols_ready = nullptr);
 
 extern int g_compare_path;
 extern int g_find_path;
-extern int g_walk_form;
+// see collection.cu
+bool probe_form_allowed(const SketchCollection &rows);
 // see include/sourmash_b200.h
 void compare_matrix(SketchCollection &rows, uint64_t r0, uint64_t nr, SketchCollection &cols, uint64_t c0, uint64_t nc,
                     int mode, uint32_t *common, uint32_t *size, double *ratio, uint64_t ld, bool out_on_device);

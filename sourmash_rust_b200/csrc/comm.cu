@@ -48,7 +48,6 @@ struct Comm {
     int rank = 0, world = 1;
     cudaStream_t stream = nullptr;            // collectives run here, beside the calling thread's compute stream
     cudaEvent_t ev_ready = nullptr, ev_done = nullptr;
-    std::vector<cudaEvent_t> ev_stage;        // one per group of a staged gather (made on first use)
     cudaStream_t build_stream = nullptr;      // the join table of a rank's own rows is built here, beside the exchange
     cudaEvent_t ev_build_go = nullptr, ev_build_done = nullptr;
     unsigned long long *d_hdr = nullptr;      // [HDR] mine + [world * HDR] everybody's
@@ -172,14 +171,6 @@ __global__ void pack_rowinfo_kernel(const uint64_t *__restrict__ offsets, const 
 
 }  // namespace
 
-// groups a uniform gather is cut into when the compare that follows can take its columns part by part
-// (1 = one ncclAllGather and one wait); SMB200_GATHER_STAGES / smgpu_gather_stages
-int g_gather_stages = [] {
-    const char *e = getenv("SMB200_GATHER_STAGES");
-    const int v = e ? atoi(e) : 1;
-    return v < 1 ? 1 : (v > 16 ? 16 : v);
-}();
-
 // ---------------------------------------------------------------------------------------------------------
 void comm_unique_id(uint8_t out[COMM_ID_BYTES]) {
     load_nccl();
@@ -228,7 +219,6 @@ void comm_destroy() {
     cudaStreamDestroy(g_comm.stream);
     cudaEventDestroy(g_comm.ev_ready);
     cudaEventDestroy(g_comm.ev_done);
-    for (cudaEvent_t e : g_comm.ev_stage) cudaEventDestroy(e);
     cudaStreamSynchronize(g_comm.build_stream);
     cudaStreamDestroy(g_comm.build_stream);
     cudaEventDestroy(g_comm.ev_build_go);
@@ -251,13 +241,11 @@ int comm_nccl_version() {
 // all-gather of a packed collection.  `meanwhile` (optional) is called once the header exchange has been queued and
 // before this thread waits for it: what it queues needs local data only and runs beside the exchange.
 // ---------------------------------------------------------------------------------------------------------
-// `arrivals` (optional, filled only for uniform rows on more than one rank): the compute stream is NOT made to wait for
-// the hashes; the caller waits for each listed event before it touches that part (collection.hpp: ColumnArrival).  With
-// g_gather_stages > 1 they travel in that many groups of point-to-point exchanges (peers by ring distance), one event
-// per group; otherwise as one ncclAllGather with one event.
+// `hashes_ready` (optional, set non-null only for uniform rows on more than one rank): the compute stream is NOT made to
+// wait for the hashes; the caller waits for that event before it touches them.
 static SketchCollection *allgather_impl(SketchCollection &local, const std::function<void()> &meanwhile,
-                                        std::vector<ColumnArrival> *arrivals = nullptr) {
-    if (arrivals) arrivals->clear();
+                                        cudaEvent_t *hashes_ready = nullptr) {
+    if (hashes_ready) *hashes_ready = nullptr;
     Comm &c = g_comm;
     Context &ctx = Context::get();
     local.finalize();  // (rows were checked strictly ascending when the local collection was made: peers do the same)
@@ -329,45 +317,12 @@ static SketchCollection *allgather_impl(SketchCollection &local, const std::func
         const uint32_t num = (uint32_t)all_shape;
         SM_CUDA(cudaEventRecord(c.ev_ready, ctx.stream));       // the output buffer is allocated (stream-ordered)
         SM_CUDA(cudaStreamWaitEvent(c.stream, c.ev_ready, 0));
-        const int G = std::min(g_gather_stages, W - 1);
-        const bool deferred = arrivals && W > 1;          // the caller waits, part by part
-        const bool grouped = deferred && g_gather_stages > 1;
-        if (grouped) {
-            // own rows: a device copy on the compute stream; peers at ring distance d, in G groups of distances -- each
-            // group is one fused NCCL kernel, and its parts can be probed while the next group is on the wire
-            uint64_t *dst = out->d_hashes.as<uint64_t>();
-            if (hashes[c.rank])
-                SM_CUDA(cudaMemcpyAsync(dst + hash_base[c.rank], local.d_hashes.p, hashes[c.rank] * 8, cudaMemcpyDeviceToDevice, ctx.stream));
-            arrivals->push_back({row_base[c.rank], row_base[c.rank] + rows[c.rank], nullptr});
-            while ((int)c.ev_stage.size() < G) {
-                cudaEvent_t e;
-                SM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                c.ev_stage.push_back(e);
-            }
-            int d = 1;
-            for (int g = 0; g < G; g++) {
-                const int d_end = 1 + (int)((uint64_t)(W - 1) * (g + 1) / G);   // distances [d, d_end)
-                SM_NCCL(g_nccl.GroupStart());
-                for (int dd = d; dd < d_end; dd++) {
-                    const int to = (c.rank + dd) % W, from = (c.rank - dd + W) % W;
-                    if (hashes[c.rank]) SM_NCCL(g_nccl.Send(local.d_hashes.p, hashes[c.rank], ncclUint64, to, c.comm, c.stream));
-                    if (hashes[from]) SM_NCCL(g_nccl.Recv(dst + hash_base[from], hashes[from], ncclUint64, from, c.comm, c.stream));
-                }
-                SM_NCCL(g_nccl.GroupEnd());
-                SM_CUDA(cudaEventRecord(c.ev_stage[g], c.stream));
-                for (int dd = d; dd < d_end; dd++) {
-                    const int from = (c.rank - dd + W) % W;
-                    arrivals->push_back({row_base[from], row_base[from] + rows[from], c.ev_stage[g]});
-                }
-                d = d_end;
-            }
-        } else {
-            SM_NCCL(g_nccl.GroupStart());
-            allgatherv(local.d_hashes.p, out->d_hashes.p, hashes, hash_base, 8, ncclUint64);
-            SM_NCCL(g_nccl.GroupEnd());
-            SM_CUDA(cudaEventRecord(c.ev_done, c.stream));
-            if (deferred) arrivals->push_back({0, n_rows, c.ev_done});
-        }
+        const bool deferred = hashes_ready && W > 1;      // the caller waits
+        SM_NCCL(g_nccl.GroupStart());
+        allgatherv(local.d_hashes.p, out->d_hashes.p, hashes, hash_base, 8, ncclUint64);
+        SM_NCCL(g_nccl.GroupEnd());
+        SM_CUDA(cudaEventRecord(c.ev_done, c.stream));
+        if (deferred) *hashes_ready = c.ev_done;
         uniform_rows_kernel<<<(unsigned)std::min<uint64_t>((n_rows + 256) / 256, 148 * 8), 256, 0, ctx.stream>>>(
             out->d_offsets.as<uint64_t>(), out->d_nums.as<uint32_t>(), n_rows, len, num);
         SM_LAUNCHED();
@@ -436,10 +391,9 @@ SketchCollection *compare_matrix_allgather(SketchCollection &local, int mode, ui
     // The hash table of the join goes over this rank's OWN rows: build it while the other ranks' rows are in flight.
     // (Only when the block will take the probe form of the join: collection.cu decides the same way.)
     const uint64_t n_rp = local.n_hashes;
-    const bool will_probe = (g_compare_path == 0 || g_compare_path == 2 || g_compare_path == 4) && n_rp > 0 && n_rp < (1ull << 31) &&
-                            local.n_rows < (1ull << 31) && !(local.probe_dense_preferred && g_compare_path == 0);
+    const bool will_probe = probe_form_allowed(local) && n_rp > 0 && n_rp < (1ull << 31) && local.n_rows < (1ull << 31);
     // (device outputs, probe form: the gathered rows may still be arriving when the block starts -- see allgather_impl)
-    std::vector<ColumnArrival> arrivals;
+    cudaEvent_t cols_ready = nullptr;
     const bool alone = !g_comm.comm || g_comm.world == 1;   // one rank: rows and columns are the same sketches
     // Queued while the headers are on their way and on a stream of its own: neither the host round trip of the headers
     // nor the transfer (whose buffers are allocated in this thread's stream order) waits for it.  Whatever happens below, this
@@ -462,26 +416,25 @@ SketchCollection *compare_matrix_allgather(SketchCollection &local, int mode, ui
             join_build.st = ctx.stream;
         }
     };
-    std::unique_ptr<SketchCollection> all(allgather_impl(local, build_table, (will_probe && out_on_device && !alone) ? &arrivals : nullptr));
+    std::unique_ptr<SketchCollection> all(allgather_impl(local, build_table, (will_probe && out_on_device && !alone) ? &cols_ready : nullptr));
     join_build.join();
-    const std::vector<ColumnArrival> *arr = arrivals.empty() ? nullptr : &arrivals;
     const uint64_t nr = local.n_rows, nc = all->n_rows;
     try {
         local.check_compatible(*all);
         if (nr != 0 && nc != 0 && ld < nc) throw_internal("ld smaller than the block width");
     } catch (...) {
-        wait_arrivals(ctx.stream, arr);   // (the gathered buffers are released in stream order)
+        if (cols_ready) SM_CUDA(cudaStreamWaitEvent(ctx.stream, cols_ready, 0));   // (the gathered buffers are released in stream order)
         throw;
     }
     if (nr == 0 || nc == 0) {
-        wait_arrivals(ctx.stream, arr);
+        if (cols_ready) SM_CUDA(cudaStreamWaitEvent(ctx.stream, cols_ready, 0));
         return all.release();
     }
     if (out_on_device) {
         try {
-            compare_block_device(local, 0, nr, alone ? local : *all, 0, nc, mode, common, size, ratio, ld, &jt, arr);
+            compare_block_device(local, 0, nr, alone ? local : *all, 0, nc, mode, common, size, ratio, ld, &jt, cols_ready);
         } catch (...) {
-            wait_arrivals(ctx.stream, arr);
+            if (cols_ready) SM_CUDA(cudaStreamWaitEvent(ctx.stream, cols_ready, 0));
             throw;
         }
         ctx.sync();

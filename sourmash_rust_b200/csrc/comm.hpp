@@ -15,7 +15,6 @@ void comm_destroy();
 int comm_rank();
 int comm_world();
 int comm_nccl_version();
-extern int g_gather_stages;  // comm.cu
 
 // every rank's rows, in rank order, on every rank (collective)
 SketchCollection *collection_allgather(SketchCollection &local);

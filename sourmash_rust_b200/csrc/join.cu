@@ -166,9 +166,7 @@ __global__ void __launch_bounds__(256) probe_group_kernel(const unsigned long lo
                                                           const uint64_t *__restrict__ po, uint64_t p0, uint64_t np, uint32_t *cmat,
                                                           uint64_t ld, unsigned long long *bitmap, uint64_t n_build,
                                                           unsigned long long *incidences, const uint32_t *__restrict__ filter,
-                                                          int log2_f, bool smem_rows, uint32_t split, uint64_t p_first) {
-    // Probing sketches p_first .. p_first + np - 1 of the block (a block whose probing side arrives in parts is
-    // probed part by part; cell ids stay those of the whole block).
+                                                          int log2_f, bool smem_rows, uint32_t split) {
     // `filter` (optional): one presence bit per build-side hash in a table small enough to stay in L2.  When
     // the two sides are unrelated collections (a query batch against an index) almost every probing hash is
     // turned away by that one bit instead of a random read in the (much larger) key table.
@@ -184,10 +182,11 @@ __global__ void __launch_bounds__(256) probe_group_kernel(const unsigned long lo
     // sketches related to the shard's rows have any hits, and one warp per sketch left most of the GPU idle while
     // those few warps walked their runs (8 GPUs, cfg3: 1 250 busy warps of 10 000).
     for (uint64_t wi = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; wi < np * split; wi += warps) {
-        const uint64_t pl = wi / split, part = wi - pl * split;
-        const uint64_t p = p_first + pl;
+        const uint64_t p = wi / split, part = wi - p * split;
         const uint64_t b0 = po[p0 + p], len = po[p0 + p + 1] - b0;
         const uint64_t b = b0 + len * part / split, e = b0 + len * (part + 1) / split;
+        // bit of (p, build sketch 0); computed here, not in the loops: there ptxas spilled in the bitmap instances
+        const uint64_t p_bits = p * n_build;
         if (s_rows) {
             for (uint32_t w = lane; w < row_words; w += 32) s_rows[w] = 0;
             __syncwarp();
@@ -237,7 +236,7 @@ __global__ void __launch_bounds__(256) probe_group_kernel(const unsigned long lo
                 if (COUNT) {
                     atomicAdd(BUILD_COLS ? &cmat[p * ld + q] : &cmat[q * ld + p], 1u);
                 } else {
-                    const uint64_t bit = p * n_build + q;
+                    const uint64_t bit = p_bits + q;
                     const unsigned long long m = 1ull << (bit & 63);
                     if (!(__ldcg(&bitmap[bit >> 6]) & m)) atomicOr(&bitmap[bit >> 6], m);  // L2 view: atomics land there
                 }
@@ -248,7 +247,7 @@ __global__ void __launch_bounds__(256) probe_group_kernel(const unsigned long lo
             for (uint32_t w = lane; w < row_words; w += 32) {
                 const unsigned long long v = s_rows[w];
                 if (v) {
-                    const uint64_t g = p * n_build + 32ull * w;
+                    const uint64_t g = p_bits + 32ull * w;
                     const unsigned sh = (unsigned)(g & 63);
                     atomicOr(&bitmap[g >> 6], v << sh);
                     if (sh > 32) atomicOr(&bitmap[(g >> 6) + 1], v >> (64 - sh));
@@ -279,7 +278,7 @@ void launch_group_fill(const uint64_t *ro, uint64_t r0, uint64_t nr, const uint3
 void launch_probe_group(bool count, bool build_cols, const unsigned long long *tkey, const uint64_t *toff, const uint32_t *grows,
                         int log2_t, const uint64_t *ph, const uint64_t *po, uint64_t p0, uint64_t np, uint32_t *cmat, uint64_t ld,
                         unsigned long long *bitmap, uint64_t n_build, unsigned long long *incidences, const uint32_t *filter,
-                        int log2_f, cudaStream_t st, uint64_t p_first) {
+                        int log2_f, cudaStream_t st) {
     if (!np) return;
     ProfScope prof(PROF_PROBE, st);
     const bool smem_rows = !count && n_build <= PROBE_SMEM_ROWS;
@@ -295,7 +294,7 @@ void launch_probe_group(bool count, bool build_cols, const unsigned long long *t
         SM_CUDA(cudaFuncSetAttribute(probe_group_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         attr_set = true;
     }
-#define SM_PROBE(C, B) probe_group_kernel<C, B><<<grid, 256, smem, st>>>(tkey, toff, grows, log2_t, ph, po, p0, np, cmat, ld, bitmap, n_build, incidences, filter, log2_f, smem_rows, split, p_first)
+#define SM_PROBE(C, B) probe_group_kernel<C, B><<<grid, 256, smem, st>>>(tkey, toff, grows, log2_t, ph, po, p0, np, cmat, ld, bitmap, n_build, incidences, filter, log2_f, smem_rows, split)
     if (count) { if (build_cols) SM_PROBE(true, true); else SM_PROBE(true, false); }
     else { if (build_cols) SM_PROBE(false, true); else SM_PROBE(false, false); }
 #undef SM_PROBE
@@ -556,132 +555,6 @@ __global__ void __launch_bounds__(256) walk_pairs_kernel(const uint64_t *__restr
         }
     }
 }
-// ---- warp-cooperative form of the same walk (both sketches of a pair together at most WW_MAX hashes) ----------------
-// One WARP per related pair.  The two sorted lists are staged in shared memory with coalesced loads; the merged
-// sequence (A before B on ties) is cut into 32 equal stretches by merge-path search (one binary search per lane); every
-// lane merges its stretch -- at most 32 steps -- and records two bit masks: which steps brought a new element of the
-// union (a B element equal to the A element just taken does not) and which were common elements.  Prefix sums over
-// the lanes give every step its rank in the union; the rule of lib.rs:470-499 -- count the common hashes among the first
-// `num` of the union -- is then a population count in the one lane where the rank crosses `num` (no second walk).
-// Same integers as the one-thread walk; what it buys is latency (shared memory instead of dependent L2 loads) and
-// parallelism when a block has few related pairs (a rank's shard on 8 GPUs: 1.25 x 10^5 pairs for 148 SMs).
-// position of the n-th (n >= 1) set bit of m
-__device__ __forceinline__ uint32_t nth_set_bit(uint32_t m, uint32_t n) {
-    uint32_t pos = 0;
-#pragma unroll
-    for (int sft = 16; sft; sft >>= 1) {
-        const uint32_t low = m & ((1u << sft) - 1u), cnt = __popc(low);
-        if (cnt < n) { n -= cnt; m >>= sft; pos += sft; } else { m = low; }
-    }
-    return pos;
-}
-constexpr uint32_t WW_MAX = 1024;                 // hashes of both sketches together
-constexpr int WW_WARPS = 8;                       // per CTA: 8 x (1024 + 8) x 8 B = 66 KB of shared memory
-__global__ void __launch_bounds__(WW_WARPS * 32) walk_pairs_warp_kernel(const uint64_t *__restrict__ pairs, uint64_t n_pairs,
-                                                                        const uint64_t *__restrict__ rh, const uint64_t *__restrict__ ro,
-                                                                        const uint32_t *__restrict__ rnum, uint64_t r0,
-                                                                        const uint64_t *__restrict__ ch, const uint64_t *__restrict__ co,
-                                                                        uint64_t c0, uint64_t nc, uint32_t *common, uint32_t *size,
-                                                                        double *ratio, uint64_t ld, const uint64_t *n_dev_a,
-                                                                        const uint64_t *n_dev_b, uint64_t nr_transposed, bool symmetric) {
-    extern __shared__ __align__(16) uint64_t s_ww[];
-    if (n_dev_a) {
-        const uint64_t nd = *n_dev_a + *n_dev_b;
-        if (nd < n_pairs) n_pairs = nd;
-    }
-    const int lane = threadIdx.x & 31;
-    uint64_t *sA = s_ww + (size_t)(threadIdx.x >> 5) * (WW_MAX + 8);
-    const uint64_t warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
-    for (uint64_t t = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; t < n_pairs; t += warps) {
-        const uint64_t cell = pairs[t];
-        uint64_t i, j;
-        if (nr_transposed) { j = cell / nr_transposed; i = cell - j * nr_transposed; }
-        else { i = cell / nc; j = cell - i * nc; }
-        if (symmetric && i > j) continue;   // (see walk_pairs_kernel)
-        const uint64_t ab = ro[r0 + i], bb = co[c0 + j];
-        const uint32_t na = (uint32_t)(ro[r0 + i + 1] - ab), nb = (uint32_t)(co[c0 + j + 1] - bb);
-        const uint32_t num = rnum ? rnum[r0 + i] : 0;
-        const uint32_t limit = num ? num : 0xFFFFFFFFu;
-        uint64_t *sB = sA + na;
-        __syncwarp();                       // the previous pair's lists are no longer read
-        for (uint32_t e = lane; e < na; e += 32) sA[e] = __ldg(rh + ab + e);
-        for (uint32_t e = lane; e < nb; e += 32) sB[e] = __ldg(ch + bb + e);
-        __syncwarp();
-        const uint32_t M = na + nb, S = (M + 31) / 32;
-        const uint32_t d0 = min(M, (uint32_t)lane * S), d1 = min(M, (uint32_t)(lane + 1) * S);
-        // merge path: ia = how many of the first d0 merged elements come from A
-        uint32_t lo = d0 > nb ? d0 - nb : 0, hi = min(d0, na);
-        while (lo < hi) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (sA[mid] <= sB[d0 - mid - 1]) lo = mid + 1; else hi = mid;
-        }
-        uint32_t ia = lo, ib = d0 - lo, umask = 0, cmask = 0;
-        for (uint32_t s = 0; s < d1 - d0; s++) {
-            const bool a_left = ia < na, b_left = ib < nb;
-            const uint64_t x = a_left ? sA[ia] : 0, y = b_left ? sB[ib] : 0;
-            if (!b_left || (a_left && x <= y)) {      // A's element (first on ties)
-                umask |= 1u << s;
-                cmask |= (uint32_t)(b_left && x == y) << s;
-                ia++;
-            } else {                                   // B's element: new to the union unless A just gave the same hash
-                umask |= (uint32_t)!(ia > 0 && sA[ia - 1] == y) << s;
-                ib++;
-            }
-        }
-        // ranks: exclusive prefix sums of the per-lane counts
-        const uint32_t u_l = __popc(umask), c_l = __popc(cmask);
-        uint32_t u_inc = u_l, c_inc = c_l;
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t uu = __shfl_up_sync(0xFFFFFFFFu, u_inc, d), cc = __shfl_up_sync(0xFFFFFFFFu, c_inc, d);
-            if (lane >= d) { u_inc += uu; c_inc += cc; }
-        }
-        const uint32_t uni = __shfl_sync(0xFFFFFFFFu, u_inc, 31), c_all = __shfl_sync(0xFFFFFFFFu, c_inc, 31);
-        const uint32_t u_before = u_inc - u_l, c_before = c_inc - c_l;
-        uint32_t c = c_all;
-        if (uni > limit) {   // only the first `limit` elements of the union count: the lane where the rank crosses it
-            const bool crossing = u_before < limit && limit <= u_inc;
-            uint32_t c_cross = 0;
-            if (crossing) {
-                const uint32_t t_last = nth_set_bit(umask, limit - u_before);   // step of the last element that still counts
-                c_cross = c_before + __popc(cmask & (t_last >= 31 ? 0xFFFFFFFFu : ((2u << t_last) - 1u)));
-            }
-            const unsigned who = __ballot_sync(0xFFFFFFFFu, crossing);
-            c = __shfl_sync(0xFFFFFFFFu, c_cross, __ffs(who) - 1);
-        }
-        if (lane == 0) {
-            const uint32_t sz = (num != 0 && uni >= num) ? num : uni;
-            const double rt = (double)c / (double)(sz > 1 ? sz : 1);
-            const size_t at = (size_t)i * ld + j;
-            if (common) common[at] = c;
-            if (size) size[at] = sz;
-            if (ratio) ratio[at] = rt;
-            if (symmetric && i != j) {
-                const size_t ta = (size_t)j * ld + i;
-                if (common) common[ta] = c;
-                if (size) size[ta] = sz;
-                if (ratio) ratio[ta] = rt;
-            }
-        }
-    }
-}
-bool walk_pairs_warp_fits(uint32_t max_row_len, uint32_t max_col_len) { return (uint64_t)max_row_len + max_col_len <= WW_MAX; }
-void launch_walk_pairs_warp(const uint64_t *pairs, uint64_t n_pairs, const uint64_t *rh, const uint64_t *ro, const uint32_t *rnum,
-                            uint64_t r0, const uint64_t *ch, const uint64_t *co, uint64_t c0, uint64_t nc, uint32_t *common,
-                            uint32_t *size, double *ratio, uint64_t ld, cudaStream_t st, const uint64_t *n_dev_a,
-                            const uint64_t *n_dev_b, uint64_t nr_transposed, bool symmetric) {
-    if (!n_pairs) return;
-    static bool attr_set = false;
-    const size_t smem = (size_t)WW_WARPS * (WW_MAX + 8) * 8;
-    if (!attr_set) {
-        SM_CUDA(cudaFuncSetAttribute(walk_pairs_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
-    ProfScope prof(PROF_WALK, st);
-    walk_pairs_warp_kernel<<<blocks_for(n_pairs * 32, WW_WARPS * 32, 148 * 12), WW_WARPS * 32, smem, st>>>(
-        pairs, n_pairs, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, n_dev_a, n_dev_b, nr_transposed, symmetric);
-    SM_LAUNCHED();
-}
-
 void launch_walk_pairs(const uint64_t *pairs, uint64_t n_pairs, const uint64_t *rh, const uint64_t *ro, const uint32_t *rnum,
                        uint64_t r0, const uint64_t *ch, const uint64_t *co, uint64_t c0, uint64_t nc, uint32_t *common,
                        uint32_t *size, double *ratio, uint64_t ld, cudaStream_t st, const uint64_t *n_dev_a,

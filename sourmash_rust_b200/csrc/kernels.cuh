@@ -184,13 +184,11 @@ void launch_group_fill(const uint64_t *ro, uint64_t r0, uint64_t nr, const uint3
                        uint32_t *tcursor, uint32_t *grows, cudaStream_t st);
 // the table was built over the rows (build_cols = false) or the columns of the block; the other side's
 // sketches [p0, p0 + np) probe it.  count: counts into cmat[r * ld + c], else related-pairs bitmap with
-// bit = probe sketch * n_build + build sketch; *incidences += hits.  p_first: probe only sketches p0 + p_first ..
-// p0 + p_first + np - 1, with the cell ids of the whole block (a probing side that arrives in parts).
+// bit = probe sketch * n_build + build sketch; *incidences += hits.
 void launch_probe_group(bool count, bool build_cols, const unsigned long long *tkey, const uint64_t *toff, const uint32_t *grows,
                         int log2_t, const uint64_t *ph, const uint64_t *po, uint64_t p0, uint64_t np, uint32_t *cmat, uint64_t ld,
                         unsigned long long *bitmap, uint64_t n_build, unsigned long long *incidences,
-                        const uint32_t *filter /*nullable: presence bits filled by launch_group_insert*/, int log2_f, cudaStream_t st,
-                        uint64_t p_first = 0);
+                        const uint32_t *filter /*nullable: presence bits filled by launch_group_insert*/, int log2_f, cudaStream_t st);
 void launch_incidences_shared(bool count, const uint64_t *keys, const uint64_t *vals, uint64_t n, uint64_t row_lo,
                               uint64_t nr, uint32_t *cmat, uint64_t ld, unsigned long long *bitmap, uint64_t nc,
                               cudaStream_t st);
@@ -239,14 +237,6 @@ void launch_stream_probe(const uint64_t *ih, const uint64_t *io, uint64_t b0, ui
 void launch_touched_hits(uint32_t *cmat, uint64_t bn, uint64_t nq, const uint64_t *row_offsets, uint64_t b0, const uint64_t *q_offsets,
                          double threshold, uint32_t *touched_bits, const uint32_t *touched_rows, unsigned long long *n_touched,
                          uint64_t *found, uint64_t cap, unsigned long long *n_found, int sm_count, cudaStream_t st);
-
-// the same walk, one WARP per pair (lists staged in shared memory, merge-path split over the lanes): for blocks whose
-// longest row + longest column fit walk_pairs_warp_fits()
-bool walk_pairs_warp_fits(uint32_t max_row_len, uint32_t max_col_len);
-void launch_walk_pairs_warp(const uint64_t *pairs, uint64_t n_pairs, const uint64_t *rh, const uint64_t *ro, const uint32_t *rnum,
-                            uint64_t r0, const uint64_t *ch, const uint64_t *co, uint64_t c0, uint64_t nc, uint32_t *common,
-                            uint32_t *size, double *ratio, uint64_t ld, cudaStream_t st, const uint64_t *n_dev_a = nullptr,
-                            const uint64_t *n_dev_b = nullptr, uint64_t nr_transposed = 0, bool symmetric = false);
 
 // dense path for full num sketches: dense u32 ranks + fixed-length walk (join.cu)
 void launch_scatter_ranks(const uint64_t *keys, const uint64_t *vals, const uint64_t *pre, uint64_t n, uint32_t L,

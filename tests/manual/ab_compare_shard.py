@@ -1,5 +1,5 @@
-"""Time one rank's row shard of the cfg3 all-vs-all matrix on one GPU for R = 1, 2, 4, 8 ranks, with and
-without the probe form of the join (smgpu_compare_path 0 / 3)."""
+"""Time one rank's row shard of the cfg3 all-vs-all matrix on one GPU for R = 1, 2, 4, 8 ranks, without and with
+the probe form of the join (smgpu_compare_path 3, and 0 / 2: chosen from the data / forced)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
@@ -16,7 +16,7 @@ for R in (1, 2, 4, 8):
     common = torch.empty((nr, N), dtype=torch.int32, device=dev); size = torch.empty_like(common)
     ratio = torch.empty((nr, N), dtype=torch.float64, device=dev)
     res = {}
-    for path in ("noprobe", "auto", "probe"):
+    for path in ("noprobe", "auto", "sparse"):
         smb.compare_path(path)
         r0 = (R // 2) * nr if R > 1 else 0
         def step():
@@ -36,7 +36,7 @@ for R in (1, 2, 4, 8):
         print("   R=%d %s: sort scope %.3f ms, join+walk scope %.3f ms" % (R, path, smb.profile_read("join_sort", True)[0],
                                                                           smb.profile_read("compare", True)[0]))
         smb.profile_enable(False)
-    print("R=%d rows %d: noprobe %.3f ms, auto %.3f ms, probe %.3f ms (checksums %d %d %d) -> whole matrix at R ranks: %.2e / %.2e pairs/s" % (
-        R, nr, res["noprobe"][0], res["auto"][0], res["probe"][0], res["noprobe"][1], res["auto"][1], res["probe"][1],
+    print("R=%d rows %d: noprobe %.3f ms, auto %.3f ms, sparse %.3f ms (checksums %d %d %d) -> whole matrix at R ranks: %.2e / %.2e pairs/s" % (
+        R, nr, res["noprobe"][0], res["auto"][0], res["sparse"][0], res["noprobe"][1], res["auto"][1], res["sparse"][1],
         N * N / (res["noprobe"][0] * 1e-3), N * N / (res["auto"][0] * 1e-3)))
 smb.compare_path("auto")

@@ -334,10 +334,10 @@ def test_host_threads_add_up():
 
 
 # ------------------------------------------------------------------------------------------------
-# the warp-cooperative form of the pair walk (join.cu: merge-path split over the lanes) against the thread form + oracle
+# the sparse path's pair walk over short sketches, num sketches cut below num, and a row shard, against the oracle
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("num,lens", [(400, (400, 401)), (0, (0, 500)), (100, (30, 300)), (512, (512, 513))])
-def test_warp_form_of_the_pair_walk(num, lens):
+def test_sparse_walk_over_short_and_partial_num_sketches(num, lens):
     r = np.random.Generator(np.random.PCG64(num + 17))
     base = [np.unique(r.integers(0, 1 << 60, size=700, dtype=np.uint64)) for _ in range(6)]
     rows, g_sk, o_sk = [], [], []
@@ -357,16 +357,13 @@ def test_warp_form_of_the_pair_walk(num, lens):
     part = smb.SketchCollection.from_sketches(g_sk[20:60])
     oc, osz = orc.compare_matrix(o_sk, o_sk)
     try:
-        for form in ("warp", "thread"):
-            smb.walk_form(form)
-            smb.compare_path("sparse")
-            common, size, ratio = smb.compare_matrix(coll, coll)             # the whole square: each unordered pair once
-            assert np.array_equal(common, oc) and np.array_equal(size, osz), form
-            assert np.array_equal(ratio, oc.astype(np.float64) / np.maximum(1, osz).astype(np.float64)), form
-            common, size, _ = smb.compare_matrix(part, coll)                 # a row shard against everything
-            assert np.array_equal(common, oc[20:60]) and np.array_equal(size, osz[20:60]), form
+        smb.compare_path("sparse")
+        common, size, ratio = smb.compare_matrix(coll, coll)             # the whole square: each unordered pair once
+        assert np.array_equal(common, oc) and np.array_equal(size, osz)
+        assert np.array_equal(ratio, oc.astype(np.float64) / np.maximum(1, osz).astype(np.float64))
+        common, size, _ = smb.compare_matrix(part, coll)                 # a row shard against everything
+        assert np.array_equal(common, oc[20:60]) and np.array_equal(size, osz[20:60])
     finally:
-        smb.walk_form("thread")
         smb.compare_path("auto")
 
 

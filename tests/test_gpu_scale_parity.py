@@ -51,23 +51,19 @@ def _built():
 
 
 @contextlib.contextmanager
-def knobs(compare=None, find=None, walk=None):
+def knobs(compare=None, find=None):
     """Sets the library's path knobs for the block and always puts them back."""
     try:
         if compare:
             smb.compare_path(compare)
         if find:
             smb.find_path(find)
-        if walk:
-            smb.walk_form(walk)
         yield
     finally:
         if compare:
             smb.compare_path("auto")
         if find:
             smb.find_path("auto")
-        if walk:
-            smb.walk_form("thread")
 
 
 def mismatch(name, got, want):
@@ -282,7 +278,7 @@ def check_padding(buf, nc, sentinel, what):
 # (a) device outputs above 2^26 cells: host-sized pair list, symmetric walk through ld > nc
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("path", ["auto", "sparse", "noprobe", "dense", "sparse+warp"])
+@pytest.mark.parametrize("path", ["auto", "sparse", "noprobe", "dense"])
 @pytest.mark.parametrize("kind", KINDS)
 def test_device_outputs_whole_square(kind, path, mode):
     import torch
@@ -291,7 +287,6 @@ def test_device_outputs_whole_square(kind, path, mode):
     assert N * N > PAIR_LIST_DEVICE_CELLS   # the sparse path sizes its pair list from the scan tail read on the host
     coll = ds.collection()
     want = expected(kind, mode)
-    compare, walk = (path.split("+") + [None])[:2]
     ld = N + 37
 
     def run(r0, nr):
@@ -299,7 +294,7 @@ def test_device_outputs_whole_square(kind, path, mode):
         s = torch.full((nr, ld), U32_SENTINEL - (1 << 32), dtype=torch.int32, device="cuda")
         r = torch.full((nr, ld), F64_SENTINEL, dtype=torch.float64, device="cuda")
         torch.cuda.synchronize()
-        with knobs(compare=compare, walk=walk):
+        with knobs(compare=path):
             smb.compare_matrix_device(coll, coll, mode, r0, nr, 0, N, c.data_ptr(), s.data_ptr(), r.data_ptr(), ld)
         out = [c.cpu().numpy().view(np.uint32), s.cpu().numpy().view(np.uint32), r.cpu().numpy()]
         del c, s, r
