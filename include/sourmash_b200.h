@@ -66,7 +66,8 @@ const uint64_t *kmerminhash_intersection_hashes(KmerMinHash *ptr, const KmerMinH
 
 /* ---- batch sketching ------------------------------------------------------------------------- */
 /* for s in 0..n_seqs: for m in 0..n_mhs: kmerminhash_add_sequence(mhs[m], buf[offsets[s]..offsets[s+1]], force)
- * (src/ffi.rs:55-70 -> src/lib.rs:252-274), sequences NOT NUL-terminated.  n_mhs <= 6.
+ * (src/ffi.rs:55-70 -> src/lib.rs:252-274), sequences NOT NUL-terminated.  n_mhs <= 6, and no sketch may
+ * appear twice in mhs (such a call is refused and changes no sketch).
  * With force == false, each sketch keeps the k-mers that precede ITS first invalid k-mer in batch
  * order and SOURMASH_ERROR_CODE_INVALID_D_N_A is recorded.
  * A device `buf` must be 16-byte aligned and readable up to offsets[n_seqs] rounded up to 16. */

@@ -679,6 +679,10 @@ struct PerSketch {
 void KmerMinHash::add_sequences(KmerMinHash *const *mhs, int n_mhs, const SeqBatch &batch, bool force) {
     if (n_mhs <= 0) return;
     if (n_mhs > 6) throw_internal("at most 6 sketches per batch call");
+    // one sketch twice would share its candidate list, device scalars and tile counter between two passes
+    for (int i = 0; i < n_mhs; i++)
+        for (int j = 0; j < i; j++)
+            if (mhs[i] == mhs[j]) throw_internal("a sketch appears more than once in one batch call");
     for (int i = 0; i < n_mhs; i++) {
         if (mhs[i]->ksize == 0) throw_internal("ksize 0");
         if (mhs[i]->is_protein && mhs[i]->ksize < 3)  // the reference reaches slice::windows(0), which panics
