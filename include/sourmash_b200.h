@@ -149,12 +149,13 @@ void smgpu_compare_matrix(SketchCollection *rows, uint64_t r0, uint64_t nr, Sket
  * matrix behind it is one smgpu_compare_matrix(mode 1) block. */
 uint64_t smgpu_scaffold_pairs(SketchCollection *c, uint64_t *pairs_first, uint64_t *pairs_second);
 /* How smgpu_compare_matrix / smgpu_linear_find walk a block: 0 (default) decides from the data --
- * an inverted index over the block's hashes finds the pairs that share at least one hash, and
- * only those are walked when the (pair, shared hash) incidences are few against the dense work;
- * 1 forces the dense tile kernel, 2 forces the inverted-index path, 3 = as 0 but with the
- * sorted-postings join instead of the hash-grouped one (the default; it builds a hash table over
- * the ROW block's hashes only, so a row shard of an all-vs-all matrix costs its share of the rows).
- * Any other value selects 0.  Results are identical. */
+ * a hash table over the smaller side of the block (a row shard of an all-vs-all matrix: its own
+ * rows, so the shard costs its share of the rows) finds the pairs that share at least one hash,
+ * and only those are walked; when the first such block over a row collection finds the
+ * (pair, shared hash) incidences many against the dense work, later blocks over those rows go
+ * to the dense kernels.  1 forces the dense kernels, 2 forces the hash-table path wherever the
+ * block fits it (a build side below 2^31 hashes).  Any other value selects 0.  Results are
+ * identical. */
 void smgpu_compare_path(int32_t path);
 /* How smgpu_linear_find counts shared hashes when a count decides the hit (containment; similarity of sketches
  * without a num): 0 (default) = an index that is large against the query batch is STREAMED once past per-slice

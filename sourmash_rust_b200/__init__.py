@@ -217,8 +217,8 @@ PROFILE_KINDS = {"sketch_k21": 0, "sketch_k31": 1, "sketch_k51": 2, "sketch_othe
 
 
 def compare_path(path="auto"):
-    """'auto' | 'dense' | 'sparse' | 'noprobe' (smgpu_compare_path)"""
-    lib().smgpu_compare_path({"auto": 0, "dense": 1, "sparse": 2, "noprobe": 3}[path])
+    """'auto' | 'dense' | 'sparse' (smgpu_compare_path)"""
+    lib().smgpu_compare_path({"auto": 0, "dense": 1, "sparse": 2}[path])
 
 
 def find_path(path="auto"):

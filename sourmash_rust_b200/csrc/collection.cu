@@ -146,7 +146,7 @@ int g_find_path = [] {
     const char *e = getenv("SMB200_FIND_PATH");
     return e ? atoi(e) : 0;
 }();
-int g_compare_path = 0;  // 0 = choose from the data, 1 = dense tile kernel, 2 = inverted-index path, 3 = inverted index without the probe form
+int g_compare_path = 0;  // 0 = choose from the data, 1 = dense kernels, 2 = probe form wherever the block fits it
 
 // The part of the probe-form decision that the compare path and the row collection make: forced sparse always probes;
 // by default a block probes unless an earlier probe over the same rows found the dense kernels the better choice.
@@ -214,9 +214,10 @@ void join_table_build(Context &ctx, JoinTable &jt, const uint64_t *bh, const uin
     jt.log2_t = log2_t; jt.log2_f = log2_f; jt.has_filter = filter != nullptr;
 }
 
-// One block of the matrix into DEVICE outputs.  Picks the sparse path (inverted index: only pairs
-// sharing a hash are walked) when the number of (pair, shared hash) incidences is small against
-// the dense work, else the dense tile kernel.  Same integers either way.
+// One block of the matrix into DEVICE outputs.  A large enough block takes the probe form of the join
+// (only pairs sharing a hash are walked) unless an earlier probe over the same rows found the dense
+// kernels the better choice; any other block is walked densely, on ranks when every sketch is full.
+// Same integers either way.
 void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, SketchCollection &cols, uint64_t c0,
                           uint64_t nc, int mode, uint32_t *common, uint32_t *size, double *ratio, uint64_t ld,
                           const JoinTable *prebuilt, cudaEvent_t cols_ready) {
@@ -233,20 +234,18 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
     const uint64_t n = n_r + n_c;
     const bool force_dense = g_compare_path == 1, force_sparse = g_compare_path == 2;
     const bool big = n > 0 && nr * nc >= 4096 && nr < (1ull << 31) && nc < (1ull << 31);
-    bool sparse = !force_dense && n > 0 && (force_sparse || big) && nr < (1ull << 31) && nc < (1ull << 31);
     // full num sketches (Jaccard): the dense walk can run on 32-bit ranks with a fixed trip count
     uint32_t L = 0, Lc = 0;
     const bool full = mode == 0 && big && block_is_full(rows, r0, nr, &L) && block_is_full(cols, c0, nc, &Lc) && L == Lc &&
                       compare_full_fits(L);
-    uint64_t *keys = nullptr, *vals = nullptr;
-    // Probe form of the join (the default sparse path): the row postings are grouped by hash in a hash
-    // table and every column hash looks its run up -- O(rows) to build, no sort, and no host round trip
-    // anywhere in the block as long as the pair list fits the cell count.  A row shard of the all-vs-all
-    // matrix therefore costs its share of the rows, which is what lets the matrix scale over GPUs; the
-    // sorted-postings join below remains for smgpu_compare_path(3) and feeds the dense rank kernel.
+    // Probe form of the join (the sparse path): the postings of the smaller side are grouped by hash in a
+    // hash table and every hash of the other side looks its run up -- O(build side) to build, no sort, and
+    // no host round trip anywhere in the block as long as the pair list fits the cell count.  A row shard
+    // of the all-vs-all matrix therefore costs its share of the rows, which is what lets the matrix scale
+    // over GPUs.  An empty build side gives an empty table: every cell is then written as unrelated.
     const uint64_t n_rp = rows.h_offsets[r0 + nr] - rows.h_offsets[r0];
     // When is the dense walk the better choice?  It costs about (|row| + |column|) / 2 steps per cell; the
-    // sparse paths cost one bitmap test per incidence plus the walk of the related pairs.  Measured at
+    // probe form costs one bitmap test per incidence plus the walk of the related pairs.  Measured at
     // num = 500 the break-even was 8 incidences per cell, i.e. one per ~60 walk steps; scale with the
     // sketch sizes (scaled sketches of 5 000 hashes: 80 per cell).
     const double avg_len = 0.5 * ((double)(rows.h_offsets[r0 + nr] - rows.h_offsets[r0]) / (double)nr + (double)n_c / (double)nc);
@@ -256,7 +255,8 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
     const uint64_t n_bp = build_cols ? n_c : n_rp, n_build = build_cols ? nc : nr;
     const uint64_t *bh = build_cols ? ch : rh, *bo = build_cols ? co : ro, *ph = build_cols ? rh : ch, *po = build_cols ? ro : co;
     const uint64_t b0 = build_cols ? c0 : r0, p0 = build_cols ? r0 : c0, n_probe = build_cols ? nr : nc;
-    const bool probe = sparse && n_bp > 0 && n_bp < (1ull << 31) && probe_form_allowed(rows);
+    const bool probe = !force_dense && n > 0 && (force_sparse || big) && nr < (1ull << 31) && nc < (1ull << 31) &&
+                       n_bp < (1ull << 31) && probe_form_allowed(rows);
     // Column hashes still in flight: the probe form with the table over the ROWS waits for them right before its probe
     // launch (what it queues first needs the rows and the column offsets only); everything else needs them now.
     cudaEvent_t probe_waits = nullptr;
@@ -336,16 +336,20 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
         }
         return;
     }
-    keys = nullptr; vals = nullptr;
-    if (sparse || (full && !force_sparse)) {
+    if (!full) {
+        launch_compare_cross(rh, ro, rnum, r0, nr, ch, co, c0, nc, mode, common, size, ratio, ld, cols.max_len, ctx.sm_count, st);
+        return;
+    }
+    // full num sketches: every hash is replaced by its rank among the block's hashes, from the sorted postings
+    // (head flags -> scan -> scatter back to sketch order)
+    ctx.join[0].reserve((n + 1) * 8);
+    ctx.join[1].reserve((n + 1) * 8);
+    uint64_t *keys = ctx.join[0].as<uint64_t>(), *vals = ctx.join[1].as<uint64_t>();
+    {
         ProfScope prof(PROF_SORT, st);
-        ctx.join[0].reserve((n + 1) * 8);
-        ctx.join[1].reserve((n + 1) * 8);
         ctx.sort_tmp_k.reserve((n + 1) * 8);
         ctx.sort_tmp_v.reserve((n + 1) * 8);
-        ctx.scan_tmp.reserve(std::max(radix_sort_scan_bytes(n), scan_tmp_bytes(std::max<uint64_t>(n, (nr * nc + 63) / 64))) + 256);
-        keys = ctx.join[0].as<uint64_t>();
-        vals = ctx.join[1].as<uint64_t>();
+        ctx.scan_tmp.reserve(std::max(radix_sort_scan_bytes(n), scan_tmp_bytes(n)) + 256);
         if (!shared) launch_postings(rh, ro, r0, nr, 0, keys, vals, st);
         launch_postings(ch, co, c0, nc, shared ? 0 : 1, keys + n_r, vals + n_r, st);
         SM_CUDA(cudaMemsetAsync(ctx.dsc(SC_TMAX), 0, 8, st));
@@ -353,67 +357,18 @@ void compare_block_device(SketchCollection &rows, uint64_t r0, uint64_t nr, Sket
         ctx.read_scalars();
         radix_sort_pairs(keys, vals, n, ctx.sort_tmp_k.as<uint64_t>(), ctx.sort_tmp_v.as<uint64_t>(),
                          std::max(1, bit_length64(ctx.h_scalars[SC_TMAX])), ctx.scan_tmp.p, ctx.scan_tmp.cap, st);
-        SM_CUDA(cudaMemsetAsync(ctx.dsc(SC_CNT), 0, 8, st));
-        if (shared) launch_count_incidences_shared(keys, vals, n, r0 - c0, nr, ctx.dsc(SC_CNT), st);
-        else launch_count_incidences(keys, vals, n, ctx.dsc(SC_CNT), st);
-        ctx.read_scalars();
-        const uint64_t incidences = ctx.h_scalars[SC_CNT];
-        if (!force_sparse && incidences > dense_if_above) sparse = false;  // mostly-related collections: the dense kernel wins
     }
-    if (!sparse && full && keys) {
-        // ranks from the sorted postings: head flags -> scan -> scatter back to sketch order
-        ctx.join[2].reserve((n + 1) * 8);
-        ctx.join[3].reserve((n + 1) * 8);
-        ctx.join[6].reserve((n + 1) * 4);
-        uint64_t *flags = ctx.join[2].as<uint64_t>(), *pre = ctx.join[3].as<uint64_t>();
-        uint32_t *ranks = ctx.join[6].as<uint32_t>();
-        launch_heads(keys, n, flags, st);
-        scan_exclusive_u64(flags, pre, n, ctx.scan_tmp.p, st);
-        launch_scatter_ranks(keys, vals, pre, n, L, n_r, ranks, st);
-        const uint32_t *rb = ranks + n_r;                                  // column sketches
-        const uint32_t *ra = shared ? rb + (r0 - c0) * (uint64_t)L : ranks;  // row sketches
-        launch_compare_full(ra, rb, L, nr, nc, common, size, ratio, ld, st);
-        return;
-    }
-    if (!sparse) {
-        launch_compare_cross(rh, ro, rnum, r0, nr, ch, co, c0, nc, mode, common, size, ratio, ld, cols.max_len, ctx.sm_count, st);
-        return;
-    }
-    ProfScope prof(PROF_COMPARE, st);
-    if (mode == 1) {
-        uint32_t *cmat = common;
-        uint64_t cld = ld;
-        if (!cmat) {
-            ctx.join[2].reserve(nr * nc * 4 + 256);
-            cmat = ctx.join[2].as<uint32_t>();
-            cld = nc;
-        }
-        SM_CUDA(cudaMemset2DAsync(cmat, cld * 4, 0, nc * 4, nr, st));
-        if (shared) launch_incidences_shared(true, keys, vals, n, r0 - c0, nr, cmat, cld, nullptr, nc, st);
-        else launch_incidences(true, keys, vals, n, cmat, cld, nullptr, nc, st);
-        launch_fill_cells(ro, rnum, r0, nr, co, c0, nc, 1, cmat, cld, common, size, ratio, ld, st);
-        return;
-    }
-    const uint64_t n_words = (nr * nc + 63) / 64;
-    ctx.join[2].reserve((n_words + 1) * 8);
-    ctx.join[3].reserve((n_words + 1) * 8);
-    ctx.join[4].reserve((n_words + 1) * 8);
-    unsigned long long *bitmap = ctx.join[2].as<unsigned long long>();
-    uint64_t *counts = ctx.join[3].as<uint64_t>(), *pre = ctx.join[4].as<uint64_t>();
-    SM_CUDA(cudaMemsetAsync(bitmap, 0, n_words * 8, st));
-    if (shared) launch_incidences_shared(false, keys, vals, n, r0 - c0, nr, nullptr, 0, bitmap, nc, st);
-    else launch_incidences(false, keys, vals, n, nullptr, 0, bitmap, nc, st);
-    launch_fill_cells(ro, rnum, r0, nr, co, c0, nc, 0, nullptr, 0, common, size, ratio, ld, st);  // as if unrelated
-    launch_popc_words(bitmap, n_words, counts, st);
-    scan_exclusive_u64(counts, pre, n_words, ctx.scan_tmp.p, st);
-    uint64_t tail[2];
-    ctx.fetch2(pre + (n_words - 1), counts + (n_words - 1), tail);
-    const uint64_t n_pairs = tail[0] + tail[1];
-    if (n_pairs) {
-        ctx.join[5].reserve((n_pairs + 1) * 8);
-        launch_expand_bits(bitmap, pre, n_words, ctx.join[5].as<uint64_t>(), st);
-        launch_walk_pairs(ctx.join[5].as<uint64_t>(), n_pairs, rh, ro, rnum, r0, ch, co, c0, nc, common, size, ratio, ld, st);
-    }
+    ctx.join[2].reserve((n + 1) * 8);
+    ctx.join[3].reserve((n + 1) * 8);
+    ctx.join[6].reserve((n + 1) * 4);
+    uint64_t *flags = ctx.join[2].as<uint64_t>(), *pre = ctx.join[3].as<uint64_t>();
+    uint32_t *ranks = ctx.join[6].as<uint32_t>();
+    launch_heads(keys, n, flags, st);
+    scan_exclusive_u64(flags, pre, n, ctx.scan_tmp.p, st);
+    launch_scatter_ranks(keys, vals, pre, n, L, n_r, ranks, st);
+    const uint32_t *rb = ranks + n_r;                                  // column sketches
+    const uint32_t *ra = shared ? rb + (r0 - c0) * (uint64_t)L : ranks;  // row sketches
+    launch_compare_full(ra, rb, L, nr, nc, common, size, ratio, ld, st);
 }
 
 void compare_matrix(SketchCollection &rows, uint64_t r0, uint64_t nr, SketchCollection &cols, uint64_t c0, uint64_t nc,

@@ -391,7 +391,7 @@ SketchCollection *compare_matrix_allgather(SketchCollection &local, int mode, ui
     // The hash table of the join goes over this rank's OWN rows: build it while the other ranks' rows are in flight.
     // (Only when the block will take the probe form of the join: collection.cu decides the same way.)
     const uint64_t n_rp = local.n_hashes;
-    const bool will_probe = probe_form_allowed(local) && n_rp > 0 && n_rp < (1ull << 31) && local.n_rows < (1ull << 31);
+    const bool will_probe = probe_form_allowed(local) && n_rp < (1ull << 31) && local.n_rows < (1ull << 31);
     // (device outputs, probe form: the gathered rows may still be arriving when the block starts -- see allgather_impl)
     cudaEvent_t cols_ready = nullptr;
     const bool alone = !g_comm.comm || g_comm.world == 1;   // one rank: rows and columns are the same sketches

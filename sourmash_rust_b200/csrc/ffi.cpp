@@ -679,7 +679,7 @@ uint64_t smgpu_scaffold_pairs(SketchCollection *c, uint64_t *pairs_first, uint64
 }
 void smgpu_fuse_multi_k(bool on) { smb200::g_fuse_multi_k = on; }
 void smgpu_find_path(int32_t path) { smb200::g_find_path = (path >= 0 && path <= 3) ? path : 0; }
-void smgpu_compare_path(int32_t path) { smb200::g_compare_path = (path >= 1 && path <= 3) ? path : 0; }
+void smgpu_compare_path(int32_t path) { smb200::g_compare_path = (path >= 1 && path <= 2) ? path : 0; }
 uint64_t smgpu_linear_find(SketchCollection *index, SketchCollection *queries, int32_t mode, double threshold,
                            uint64_t *hit_offsets, uint64_t *hits, uint64_t hits_cap) {
     return landingpad<uint64_t>([&]() {

@@ -1,11 +1,12 @@
-// join.cu -- sparse all-vs-all: find the sketch pairs that share at least one hash with an
-// inverted index (sort all (hash, sketch) postings, walk the runs of equal hashes), so that the
-// merge walk of the reference (Intersection, src/lib.rs:515-544, inside intersection_size,
-// lib.rs:470-499) only runs for related pairs.  Unrelated pairs have common = 0 and
-// size = min(num, |A| + |B|) by definition, no walk needed.  For the untruncated intersection
-// (count_common, lib.rs:428-436; Leaf containment, index.rs:146-160) the postings walk yields
-// the counts directly.  Results are the same integers as the dense kernel's; which path runs is
-// decided from the number of (pair, shared hash) incidences.
+// join.cu -- sparse all-vs-all: find the sketch pairs that share at least one hash with a hash
+// table grouped by hash (the probe form: the postings of one side of the block are grouped by hash,
+// every hash of the other side looks its run up), so that the merge walk of the reference
+// (Intersection, src/lib.rs:515-544, inside intersection_size, lib.rs:470-499) only runs for related
+// pairs.  Unrelated pairs have common = 0 and size = min(num, |A| + |B|) by definition, no walk
+// needed.  For the untruncated intersection (count_common, lib.rs:428-436; Leaf containment,
+// index.rs:146-160) the probe yields the counts directly.  Results are the same integers as the dense
+// kernels'.  Sorted (hash, sketch) postings serve only the dense kernel of full num sketches (end of
+// this file), which walks ranks of the hashes instead of the hashes.
 #include <algorithm>
 
 #include "device.hpp"
@@ -39,36 +40,6 @@ void launch_postings(const uint64_t *hashes, const uint64_t *offsets, uint64_t f
                      uint64_t *keys, uint64_t *vals, cudaStream_t st) {
     if (!n_rows) return;
     postings_kernel<<<blocks_for(n_rows * 32, 256, 148 * 16), 256, 0, st>>>(hashes, offsets, first, n_rows, side, keys, vals);
-    SM_LAUNCHED();
-}
-
-// number of (row posting, column posting) incidences = sum over runs of equal hashes of
-// (row-side members) x (column-side members); the head of each run counts its run
-__global__ void __launch_bounds__(256) count_incidences_kernel(const uint64_t *__restrict__ keys,
-                                                               const uint64_t *__restrict__ vals, uint64_t n,
-                                                               unsigned long long *out) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    const uint64_t n_round = (n + 31) / 32 * 32;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += stride) {
-        unsigned long long local = 0;
-        if (i < n) {
-            const uint64_t key = keys[i];
-            if (i == 0 || keys[i - 1] != key) {
-                unsigned long long mr = 0, mc = 0;
-                for (uint64_t j = i; j < n && keys[j] == key; j++) {
-                    if (vals[j] >> 63) mc++; else mr++;
-                }
-                local = mr * mc;
-            }
-        }
-        for (int d = 16; d; d >>= 1) local += __shfl_xor_sync(0xFFFFFFFFu, local, d);
-        if ((threadIdx.x & 31) == 0 && local) atomicAdd(out, local);
-    }
-}
-void launch_count_incidences(const uint64_t *keys, const uint64_t *vals, uint64_t n, unsigned long long *out,
-                             cudaStream_t st) {
-    if (!n) return;
-    count_incidences_kernel<<<blocks_for(n, 256, 148 * 16), 256, 0, st>>>(keys, vals, n, out);
     SM_LAUNCHED();
 }
 
@@ -298,114 +269,6 @@ void launch_probe_group(bool count, bool build_cols, const unsigned long long *t
     if (count) { if (build_cols) SM_PROBE(true, true); else SM_PROBE(true, false); }
     else { if (build_cols) SM_PROBE(false, true); else SM_PROBE(false, false); }
 #undef SM_PROBE
-    SM_LAUNCHED();
-}
-
-// One postings set for both sides (rows and columns come from the same collection and the row range
-// lies inside the column range): posting value = column-local sketch id << 32 | position; a posting is
-// also a row posting when its sketch lies in [row_lo, row_lo + nr) (column-local ids).  Each posting
-// walks forward over its run and handles both ordered pairs it forms with every later member, plus
-// the pair with itself.
-template <bool COUNT>
-__global__ void __launch_bounds__(256) incidences_shared_kernel(const uint64_t *__restrict__ keys,
-                                                                const uint64_t *__restrict__ vals, uint64_t n,
-                                                                uint64_t row_lo, uint64_t nr, uint32_t *cmat, uint64_t ld,
-                                                                unsigned long long *bitmap, uint64_t nc) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    auto hit = [&](uint64_t r, uint64_t c) {
-        if (COUNT) {
-            atomicAdd(&cmat[r * ld + c], 1u);
-        } else {
-            const uint64_t bit = r * nc + c;
-            const unsigned long long m = 1ull << (bit & 63);
-            if (!(bitmap[bit >> 6] & m)) atomicOr(&bitmap[bit >> 6], m);
-        }
-    };
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const uint64_t key = keys[i];
-        const uint64_t ci = vals[i] >> 32;
-        const bool i_row = ci >= row_lo && ci - row_lo < nr;
-        if (i_row) hit(ci - row_lo, ci);
-        for (uint64_t j = i + 1; j < n && keys[j] == key; j++) {
-            const uint64_t cj = vals[j] >> 32;
-            if (i_row) hit(ci - row_lo, cj);
-            if (cj >= row_lo && cj - row_lo < nr) hit(cj - row_lo, ci);
-        }
-    }
-}
-void launch_incidences_shared(bool count, const uint64_t *keys, const uint64_t *vals, uint64_t n, uint64_t row_lo,
-                              uint64_t nr, uint32_t *cmat, uint64_t ld, unsigned long long *bitmap, uint64_t nc,
-                              cudaStream_t st) {
-    if (!n) return;
-    if (count) incidences_shared_kernel<true><<<blocks_for(n, 256, 148 * 32), 256, 0, st>>>(keys, vals, n, row_lo, nr, cmat, ld, bitmap, nc);
-    else incidences_shared_kernel<false><<<blocks_for(n, 256, 148 * 32), 256, 0, st>>>(keys, vals, n, row_lo, nr, cmat, ld, bitmap, nc);
-    SM_LAUNCHED();
-}
-// incidences of the shared-postings form: per run of m members of which mr are rows: mr * m
-__global__ void __launch_bounds__(256) count_incidences_shared_kernel(const uint64_t *__restrict__ keys,
-                                                                      const uint64_t *__restrict__ vals, uint64_t n,
-                                                                      uint64_t row_lo, uint64_t nr, unsigned long long *out) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    const uint64_t n_round = (n + 31) / 32 * 32;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_round; i += stride) {
-        unsigned long long local = 0;
-        if (i < n) {
-            const uint64_t key = keys[i];
-            if (i == 0 || keys[i - 1] != key) {
-                unsigned long long m = 0, mr = 0;
-                for (uint64_t j = i; j < n && keys[j] == key; j++) {
-                    const uint64_t c = vals[j] >> 32;
-                    m++;
-                    mr += (c >= row_lo && c - row_lo < nr);
-                }
-                local = mr * m;
-            }
-        }
-        for (int d = 16; d; d >>= 1) local += __shfl_xor_sync(0xFFFFFFFFu, local, d);
-        if ((threadIdx.x & 31) == 0 && local) atomicAdd(out, local);
-    }
-}
-void launch_count_incidences_shared(const uint64_t *keys, const uint64_t *vals, uint64_t n, uint64_t row_lo, uint64_t nr,
-                                    unsigned long long *out, cudaStream_t st) {
-    if (!n) return;
-    count_incidences_shared_kernel<<<blocks_for(n, 256, 148 * 16), 256, 0, st>>>(keys, vals, n, row_lo, nr, out);
-    SM_LAUNCHED();
-}
-
-// Sorted postings (stable sort of [row postings, column postings]: inside a run of equal hashes the
-// row side comes first).  Every row posting walks forward over its run and, for each column posting,
-//   COUNT : atomicAdd(cmat[r * ld + c], 1)        (untruncated |A n B|)
-//   !COUNT: atomicOr on the related-pair bitmap   (bit r * nc + c)
-template <bool COUNT>
-__global__ void __launch_bounds__(256) incidences_kernel(const uint64_t *__restrict__ keys,
-                                                         const uint64_t *__restrict__ vals, uint64_t n,
-                                                         uint32_t *cmat, uint64_t ld, unsigned long long *bitmap,
-                                                         uint64_t nc) {
-    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const uint64_t v = vals[i];
-        if (v >> 63) continue;  // column posting
-        const uint64_t key = keys[i];
-        const uint64_t r = (v >> 32) & 0x7FFFFFFFull;
-        for (uint64_t j = i + 1; j < n && keys[j] == key; j++) {
-            const uint64_t w = vals[j];
-            if (!(w >> 63)) continue;  // another row posting of the run
-            const uint64_t c = (w >> 32) & 0x7FFFFFFFull;
-            if (COUNT) {
-                atomicAdd(&cmat[r * ld + c], 1u);
-            } else {
-                const uint64_t bit = r * nc + c;
-                const unsigned long long m = 1ull << (bit & 63);
-                if (!(bitmap[bit >> 6] & m)) atomicOr(&bitmap[bit >> 6], m);  // test first: most incidences repeat a pair
-            }
-        }
-    }
-}
-void launch_incidences(bool count, const uint64_t *keys, const uint64_t *vals, uint64_t n, uint32_t *cmat, uint64_t ld,
-                       unsigned long long *bitmap, uint64_t nc, cudaStream_t st) {
-    if (!n) return;
-    if (count) incidences_kernel<true><<<blocks_for(n, 256, 148 * 32), 256, 0, st>>>(keys, vals, n, cmat, ld, bitmap, nc);
-    else incidences_kernel<false><<<blocks_for(n, 256, 148 * 32), 256, 0, st>>>(keys, vals, n, cmat, ld, bitmap, nc);
     SM_LAUNCHED();
 }
 

@@ -169,10 +169,6 @@ void launch_compact_indices(const uint64_t *flags, const uint64_t *pre, uint64_t
 // ---- join.cu: sparse all-vs-all through an inverted index (see the file header) ----------------
 void launch_postings(const uint64_t *hashes, const uint64_t *offsets, uint64_t first, uint64_t n_rows, uint64_t side,
                      uint64_t *keys, uint64_t *vals, cudaStream_t st);
-void launch_count_incidences(const uint64_t *keys, const uint64_t *vals, uint64_t n, unsigned long long *out,
-                             cudaStream_t st);
-void launch_incidences(bool count, const uint64_t *keys, const uint64_t *vals, uint64_t n, uint32_t *cmat, uint64_t ld,
-                       unsigned long long *bitmap, uint64_t nc, cudaStream_t st);
 void launch_max_u64(const uint64_t *keys, uint64_t n, unsigned long long *out, cudaStream_t st);
 // probe form of the join (join.cu): row postings grouped by hash in a hash table of 2^log2_t (+1) slots
 //   tkey  (2^log2_t + 1) u64, preset to ~0;  tcount (2^log2_t + 2) u64, zeroed;  tcursor (2^log2_t + 1) u32, zeroed
@@ -189,11 +185,6 @@ void launch_probe_group(bool count, bool build_cols, const unsigned long long *t
                         int log2_t, const uint64_t *ph, const uint64_t *po, uint64_t p0, uint64_t np, uint32_t *cmat, uint64_t ld,
                         unsigned long long *bitmap, uint64_t n_build, unsigned long long *incidences,
                         const uint32_t *filter /*nullable: presence bits filled by launch_group_insert*/, int log2_f, cudaStream_t st);
-void launch_incidences_shared(bool count, const uint64_t *keys, const uint64_t *vals, uint64_t n, uint64_t row_lo,
-                              uint64_t nr, uint32_t *cmat, uint64_t ld, unsigned long long *bitmap, uint64_t nc,
-                              cudaStream_t st);
-void launch_count_incidences_shared(const uint64_t *keys, const uint64_t *vals, uint64_t n, uint64_t row_lo, uint64_t nr,
-                                    unsigned long long *out, cudaStream_t st);
 void launch_popc_words(const unsigned long long *bitmap, uint64_t n_words, uint64_t *counts, cudaStream_t st);
 void launch_expand_bits(const unsigned long long *bitmap, const uint64_t *pre, uint64_t n_words, uint64_t *pairs,
                         cudaStream_t st, uint64_t cap = ~0ull);

@@ -20,7 +20,7 @@ sk = []
 for i in range(40):
     m = smb.KmerMinHash(100, 21, False, 42, 0, False); m.add_sequence(g[i * 300:i * 300 + 6000]); sk.append(m)
 coll = smb.SketchCollection.from_sketches(sk)
-for path in ("auto", "noprobe", "dense"):
+for path in ("auto", "dense"):
     smb.compare_path(path)
     cm, sz, r = smb.compare_matrix(coll, coll, "compare")
     cm2, _, _ = smb.compare_matrix(coll, coll, "containment", r0=3, nr=9)

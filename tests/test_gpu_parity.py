@@ -2,6 +2,7 @@
 include/sourmash_b200.h) is compared bit-for-bit with the CPU oracle (oracle/oracle.c, a
 restatement of the reference pinned by tests/test_oracle.py) on the same inputs, and with the
 reference's own known-answer tests and fixtures."""
+import contextlib
 import json
 
 import numpy as np
@@ -544,6 +545,21 @@ def compare_path(request):
     smb.compare_path("auto")
 
 
+@contextlib.contextmanager
+def scope_counts(*kinds):
+    """Launches per profiler scope inside the block (profiling on: one stream): got[kind] afterwards."""
+    for kd in kinds:
+        smb.profile_read(kd, reset=True)
+    got = {}
+    smb.profile_enable(True)
+    try:
+        yield got
+    finally:
+        smb.profile_enable(False)
+        for kd in kinds:
+            got[kd] = smb.profile_read(kd, reset=True)[1]
+
+
 @pytest.mark.parametrize("compare_path", ["auto", "dense", "sparse"], indirect=True)
 @pytest.mark.parametrize("num,n_hashes,mx", [(500, 500, 0), (0, 1200, MAX_HASH_1000 * 50), (100, 130, 0)])
 def test_compare_matrix_vs_oracle(num, n_hashes, mx, compare_path):
@@ -583,17 +599,19 @@ def test_compare_matrix_vs_oracle(num, n_hashes, mx, compare_path):
                 assert got[q] == orc.linear_find(o_sk, o_sk[q], mode, thr)
 
 
-@pytest.mark.parametrize("compare_path", ["auto", "sparse", "noprobe", "dense"], indirect=True)
+@pytest.mark.parametrize("compare_path", ["auto", "sparse", "dense"], indirect=True)
 @pytest.mark.parametrize("num,n_hashes,mx", [(400, 400, 0), (0, 900, MAX_HASH_1000 * 50)])
 def test_compare_row_shards_and_query_batches(num, n_hashes, mx, compare_path):
     """Row blocks much narrower than the column block -- a rank's shard of the all-vs-all matrix, a query
-    batch against an index -- take the probe form of the join (only the row postings are sorted); every
+    batch against an index -- take the probe form of the join (a hash table over the smaller side); every
     path must give the oracle's integers."""
     rows = _planted_rows(240, n_hashes, 91 + num, mx or None)
     if num:
         rows = [r[:num] for r in rows]
     rows[50] = rows[50][:0]
     rows[51] = rows[51][:2]
+    for i in range(140, 160):  # a shard of empty sketches only
+        rows[i] = rows[i][:0]
     g_sk, o_sk = [], []
     for r in rows:
         g, o = pair(num, 31, mx)
@@ -612,6 +630,19 @@ def test_compare_row_shards_and_query_batches(num, n_hashes, mx, compare_path):
         common, size, ratio = smb.compare_matrix(coll, coll, "containment", r0=r0, nr=nr)
         assert np.array_equal(common, occ[r0:r0 + nr])
         assert np.array_equal(size, np.repeat(lens[r0:r0 + nr, None], len(rows), 1))
+    # The shard of empty rows: the probe form builds an empty table and writes every cell as unrelated.  As the
+    # first block of its collection it takes the probe form on "auto" too (20 x 240 cells: past the size threshold).
+    r0, nr = 140, 20
+    assert nr * len(rows) >= 4096
+    fresh = smb.SketchCollection.from_sketches(g_sk)
+    with scope_counts("compare_probe") as probed:
+        common, size, ratio = smb.compare_matrix(fresh, fresh, "compare", r0=r0, nr=nr)
+        ccommon, csize, _ = smb.compare_matrix(fresh, fresh, "containment", r0=r0, nr=nr)
+    assert np.array_equal(common, oc[r0:r0 + nr]) and np.array_equal(size, osz[r0:r0 + nr])
+    assert np.array_equal(ratio, oc[r0:r0 + nr].astype(np.float64) / np.maximum(1, osz[r0:r0 + nr]).astype(np.float64))
+    assert np.array_equal(ccommon, occ[r0:r0 + nr]) and not csize.any()
+    if compare_path != "dense":
+        assert probed["compare_probe"] == 2
     # a separate (small) query collection as the ROW side, the index as columns, and the other way round
     queries = smb.SketchCollection.from_sketches(g_sk[100:120])
     common, size, ratio = smb.compare_matrix(queries, coll, "compare")
@@ -648,12 +679,12 @@ def test_compare_mostly_unrelated_clusters(compare_path):
     assert np.array_equal(ccommon[:200, :200], orc.count_common_matrix(osk[:200], osk[:200]))
     assert (csize == 500).all() and np.array_equal(cratio, ccommon / 500.0)
     assert common[16, 17] == 500 and ratio[16, 17] == 1.0
-    # row-sharded block of the same collection (one postings set serves both sides) ...
+    # row-sharded block of the same collection (the rows are part of the columns) ...
     c2, s2, r2 = smb.compare_matrix(coll, coll, "compare", r0=100, nr=150, c0=0, nc=N)
     assert np.array_equal(c2, oc[100:250]) and np.array_equal(s2, osz[100:250])
     c2, s2, r2 = smb.compare_matrix(coll, coll, "containment", r0=100, nr=150, c0=50, nc=300)
     assert np.array_equal(c2, ccommon[100:250, 50:350])
-    # ... and a row range that sticks out of the column range (two postings sets)
+    # ... and a row range that sticks out of the column range
     c2, s2, r2 = smb.compare_matrix(coll, coll, "compare", r0=0, nr=300, c0=200, nc=300)
     assert np.array_equal(c2, oc[0:300, 200:500]) and np.array_equal(r2, (oc / np.maximum(1, osz))[0:300, 200:500])
 
@@ -688,6 +719,35 @@ def test_compare_mostly_related_full_sketches(compare_path):
     assert np.array_equal(c2, oc[33:103])
     c2, s2, r2 = smb.compare_matrix(coll, other, "compare", r0=5, nr=100, c0=0, nc=70)
     assert np.array_equal(c2, oc[5:105, 40:110]) and np.array_equal(r2, (oc / np.maximum(1, osz))[5:105, 40:110])
+
+
+@pytest.mark.parametrize("compare_path", ["auto"], indirect=True)
+def test_compare_mostly_related_scaled_sketches(compare_path):
+    # one big family of scaled sketches of different lengths: the first block over the rows probes and finds the
+    # dense walk the better choice; every later block over the same rows goes to the dense kernel directly
+    r = np.random.Generator(np.random.PCG64(13))
+    N, mx = 150, MAX_HASH_1000 * 50
+    root = np.unique(r.integers(0, mx, size=2000, dtype=np.uint64))
+    rows = []
+    for i in range(N):
+        kept = root[r.random(root.size) < (0.5, 0.7, 0.9)[i % 3]]
+        rows.append(np.unique(np.concatenate([kept, r.integers(0, mx, size=int(r.integers(10, 600)), dtype=np.uint64)])))
+    gs, osk = [], []
+    for row in rows:
+        g, o = pair(0, 31, mx)
+        g.set_mins(row); o.add_many(row)
+        gs.append(g); osk.append(o)
+    assert len({len(row) for row in rows}) > 1
+    coll = smb.SketchCollection.from_sketches(gs)
+    oc, osz = orc.compare_matrix(osk, osk, 4)
+    with scope_counts("compare_probe") as first:
+        common, size, ratio = smb.compare_matrix(coll, coll, "compare")
+    assert np.array_equal(common, oc) and np.array_equal(size, osz) and np.array_equal(ratio, oc / np.maximum(1, osz))
+    assert first["compare_probe"] == 1
+    with scope_counts("compare_probe", "join_sort", "compare") as again:
+        common, size, ratio = smb.compare_matrix(coll, coll, "compare")
+    assert np.array_equal(common, oc) and np.array_equal(size, osz) and np.array_equal(ratio, oc / np.maximum(1, osz))
+    assert again["compare_probe"] == 0 and again["join_sort"] == 0 and again["compare"] >= 1
 
 
 def test_scaffold_leaf_pairing():  # SURVEY 8(f) rank 2: src/index/sbt.rs:356-381

@@ -278,7 +278,7 @@ def check_padding(buf, nc, sentinel, what):
 # (a) device outputs above 2^26 cells: host-sized pair list, symmetric walk through ld > nc
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("path", ["auto", "sparse", "noprobe", "dense"])
+@pytest.mark.parametrize("path", ["auto", "sparse", "dense"])
 @pytest.mark.parametrize("kind", KINDS)
 def test_device_outputs_whole_square(kind, path, mode):
     import torch
@@ -310,7 +310,7 @@ def test_device_outputs_whole_square(kind, path, mode):
 # (b) host outputs over three or more 2^25-cell row blocks: double buffering, strided copies, output subsets
 # ------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("mode", MODES)
-@pytest.mark.parametrize("path", ["auto", "sparse", "noprobe", "dense"])
+@pytest.mark.parametrize("path", ["auto", "sparse", "dense"])
 @pytest.mark.parametrize("kind", KINDS)
 def test_host_outputs_row_blocks(kind, path, mode):
     ds = square(kind)
@@ -650,7 +650,7 @@ def test_edge_values_add_many(abund):
             assert g.mins_np()[-1] == EDGE[-1] and g.mins_np()[0] == 0
 
 
-@pytest.mark.parametrize("path", ["auto", "sparse", "noprobe", "dense"])
+@pytest.mark.parametrize("path", ["auto", "sparse", "dense"])
 @pytest.mark.parametrize("kind", list(EDGE_KINDS))
 def test_edge_values_compare_matrix(kind, path):
     rows, gs, os_ = edge_case(kind)
