@@ -171,17 +171,35 @@ KB_HD void extract2_end(const uint32_t *w, uint32_t s, uint32_t (&e)[KmerGeom<K>
 // strands: with comp(c) = ~c, BE(fw) = ~E(rc) and BE(rc) = ~E(fw), so fw <lex rc <=> E(fw) < E(rc).
 template <int K>
 KB_HD bool canonical_is_fw(const uint32_t (&ef)[KmerGeom<K>::NE], const uint32_t (&er)[KmerGeom<K>::NE]) {
-    // multi-word unsigned compare, most significant words first, as 64-bit pieces (ISETP + ISETP.EX);
-    // ties -> rc, as the reference's `else` arm (identical bytes anyway)
+    // multi-word unsigned compare: up to two words as one 64-bit compare (ISETP + ISETP.EX), more as a borrow
+    // chain on the device; ties -> rc, as the reference's `else` arm (identical bytes anyway)
     constexpr int NE = KmerGeom<K>::NE;
     if (NE == 1) return ef[0] < er[0];
     if (NE == 2) return (((uint64_t)ef[1] << 32) | ef[0]) < (((uint64_t)er[1] << 32) | er[0]);
+#if defined(__CUDA_ARCH__)
+    // one borrow chain ef - er over all words (missing top words are 0 - 0, which pass the borrow on): fw < rc
+    // exactly when it borrows out of the top word.  Replaces a compare / compare / select per word.
+    static_assert(NE <= 4, "borrow chain spelled for up to four words");
+    uint32_t f[4] = {0, 0, 0, 0}, r[4] = {0, 0, 0, 0}, borrow;
+#pragma unroll
+    for (int j = 0; j < NE; j++) { f[j] = ef[j]; r[j] = er[j]; }
+    asm("{\n\t.reg .u32 t;\n\t"
+        "sub.cc.u32 t, %1, %5;\n\t"
+        "subc.cc.u32 t, %2, %6;\n\t"
+        "subc.cc.u32 t, %3, %7;\n\t"
+        "subc.cc.u32 t, %4, %8;\n\t"
+        "subc.u32 %0, 0, 0;\n\t}"
+        : "=r"(borrow)
+        : "r"(f[0]), "r"(f[1]), "r"(f[2]), "r"(f[3]), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]));
+    return borrow != 0;
+#else
     bool lt = false;
 #pragma unroll
     for (int j = 0; j < NE; j++) {  // least significant word first; later words override
         if (ef[j] != er[j]) lt = ef[j] < er[j];
     }
     return lt;
+#endif
 }
 
 // K ASCII bytes starting at byte `start` of a byte stream viewed as words (readable up to

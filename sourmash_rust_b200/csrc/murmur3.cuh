@@ -49,23 +49,13 @@ SM_HD uint64_t mm_mulc(uint64_t x) {
     return x * C;
 #endif
 }
-// x * 5 + ADD
+// x * 5 + ADD.  On the device this compiles to IMAD.WIDE.U32 with the constant as a 64-bit addend + IMAD +
+// IMAD.IADD: the fewest issue slots of the forms tried, which is what the sketch kernels are bound by.  A
+// `mul.wide.u32` + `mad.lo` + `add.cc/addc` form and an ALU shift-add form take fewer FMA-heavy cycles by the
+// static model but no fewer instructions, and measured no faster (DESIGN 4.1).
 template <uint32_t ADD>
 SM_HD uint64_t mm_mul5add(uint64_t x) {
-#if defined(__CUDA_ARCH__) && defined(MM_MUL5_WIDE)
-    uint64_t r;
-    asm("{\n\t.reg .u32 lo, hi, rl, rh;\n\t.reg .u64 t;\n\t"
-        "mov.b64 {lo, hi}, %1;\n\t"
-        "mad.wide.u32 t, lo, 5, %2;\n\t"
-        "mov.b64 {rl, rh}, t;\n\t"
-        "mad.lo.u32 rh, hi, 5, rh;\n\t"
-        "mov.b64 %0, {rl, rh};\n\t}"
-        : "=l"(r)
-        : "l"(x), "l"((uint64_t)ADD));
-    return r;
-#else
     return x * 5 + ADD;
-#endif
 }
 template <int R>
 SM_HD uint64_t mm_rotl64(uint64_t x) {
@@ -94,14 +84,16 @@ SM_HD uint64_t mm_xorshift33(uint64_t k) {
     return k ^ (k >> 33);
 #endif
 }
-SM_HD uint64_t mm_fmix64(uint64_t k) {
+// fmix64 without its last xorshift33, which leaves the high word as it is: the sketch kernels test the high words
+// first and finish the hash only for the rare windows that may pass (murmur3_h1_words_parts)
+SM_HD uint64_t mm_fmix64_pre(uint64_t k) {
     k = mm_xorshift33(k);
     k = mm_mulc<0xff51afd7ed558ccdULL>(k);
     k = mm_xorshift33(k);
     k = mm_mulc<0xc4ceb9fe1a85ec53ULL>(k);
-    k = mm_xorshift33(k);
     return k;
 }
+SM_HD uint64_t mm_fmix64(uint64_t k) { return mm_xorshift33(mm_fmix64_pre(k)); }
 
 SM_HD uint64_t mm_mix_k1(uint64_t k1) {
     k1 = mm_mulc<MM_C1>(k1); k1 = mm_rotl64<31>(k1); k1 = mm_mulc<MM_C2>(k1);
@@ -147,9 +139,10 @@ SM_HD uint64_t murmur3_h1_bytes(const uint8_t *data, uint64_t len, uint64_t seed
     return mm_final_h1(h1, h2, len);
 }
 
-// K bytes held in ceil(K/4) little-endian 32-bit words; fully unrolled.
+// K bytes held in ceil(K/4) little-endian 32-bit words; fully unrolled.  Returns the hash in two parts,
+// h1 = mm_xorshift33(a) + mm_xorshift33(b) (mod 2^64), where the high words of a and b are those of the two addends.
 template <int K>
-SM_HD uint64_t murmur3_h1_words(const uint32_t *w, uint64_t seed) {
+SM_HD void murmur3_h1_words_parts(const uint32_t *w, uint64_t seed, uint64_t &a, uint64_t &b) {
     constexpr int NB = K / 16;
     constexpr int REM = K % 16;
     uint64_t h1 = seed, h2 = seed;
@@ -169,7 +162,15 @@ SM_HD uint64_t murmur3_h1_words(const uint32_t *w, uint64_t seed) {
         const uint64_t k1 = ((uint64_t)hi << 32) | w[4 * NB + 0];
         h1 ^= mm_mix_k1(k1);
     }
-    return mm_final_h1(h1, h2, (uint64_t)K);
+    h1 ^= (uint64_t)K; h2 ^= (uint64_t)K;
+    h1 += h2; h2 += h1;
+    a = mm_fmix64_pre(h1); b = mm_fmix64_pre(h2);
+}
+template <int K>
+SM_HD uint64_t murmur3_h1_words(const uint32_t *w, uint64_t seed) {
+    uint64_t a, b;
+    murmur3_h1_words_parts<K>(w, seed, a, b);
+    return mm_xorshift33(a) + mm_xorshift33(b);
 }
 
 }  // namespace smb200

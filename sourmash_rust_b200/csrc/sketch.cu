@@ -317,6 +317,13 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
     const uint32_t *qsb = sbad + (tid >> 5);
     uint32_t mb = 1u << (tid & 31);
     asm("" : "+r"(mb));  // opaque: keeps the validity test a single LOP3 against a resident mask
+    // Prefilter on the high words.  The hash is xs(a) + xs(b) (murmur3_h1_words_parts) and xs keeps the high word, so
+    // its high word is hi(a) + hi(b) + carry, carry 0 or 1: h <= thr needs s = hi(a) + hi(b) (mod 2^32) in
+    // [0, hi(thr)] or s = 2^32 - 1, i.e. s + 1 <= hi(thr) + 1 (mod 2^32; every s when hi(thr) = 2^32 - 1).  Only the
+    // windows that pass finish the hash (two xorshifts, a 64-bit add and compare) and test h <= thr exactly.
+    const uint32_t thr_hi = (uint32_t)(thr >> 32);
+    uint32_t lim = thr_hi == 0xFFFFFFFFu ? thr_hi : thr_hi + 1u;
+    asm("" : "+r"(lim));  // opaque: computed once, not again per window
     // running word pointers: stepped once per UNROLL windows, constant offsets inside
 #pragma unroll 1
     for (int r = 0; r < SK_TILE / SK_THREADS; r += UNROLL) {
@@ -336,8 +343,12 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
 #else
             extractAw<K>(pa, use_fw ? sfa : sra, kw);
 #endif
-            const uint64_t h = murmur3_h1_words<K>(kw, sb.seed);
-            append_survivor(valid && h <= thr, h, t0 + (uint32_t)((r + u) * SK_THREADS), sb, out);
+            uint64_t a, b;
+            murmur3_h1_words_parts<K>(kw, sb.seed, a, b);
+            if (valid & ((uint32_t)(a >> 32) + (uint32_t)(b >> 32) + 1u <= lim)) {  // `&`: one test, no early branch
+                const uint64_t h = mm_xorshift33(a) + mm_xorshift33(b);
+                append_survivor(h <= thr, h, t0 + (uint32_t)((r + u) * SK_THREADS), sb, out);
+            }
         }
         qf2 += UNROLL * (SK_THREADS / 16); qr2 -= UNROLL * (SK_THREADS / 16);
         qfa += UNROLL * (SK_THREADS / 4);  qra -= UNROLL * (SK_THREADS / 4);
