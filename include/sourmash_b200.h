@@ -122,6 +122,24 @@ SketchCollection *smgpu_collection_from_csr(const uint64_t *hashes /*[host|devic
 SketchCollection *smgpu_sketch_collection(const char *buf /*[host|device]*/, const uint64_t *offsets /*[host|device], n_seqs + 1 */,
                                           uint64_t n_seqs, uint32_t num, uint32_t ksize, uint64_t seed, uint64_t max_hash,
                                           bool on_device);
+/* One collection per template, each holding one fresh sketch per sequence:
+ *   for s in 0..n_seqs: for m in 0..n_templates:
+ *     mh = kmerminhash_new(num_m, ksize_m, is_protein_m, seed_m, max_hash_m, false);
+ *     kmerminhash_add_sequence(mh, buf[offsets[s]..offsets[s+1]], force = true);
+ *     smgpu_collection_push(out[m], mh)
+ * in ONE pass over the batch: a host batch crosses PCIe once, DNA templates with distinct k in {21, 31, 51}
+ * and one seed share the fused launch of smgpu_fuse_multi_k, and protein templates share one six-frame
+ * translation of the batch.  out[m] equals smgpu_sketch_collection with template m's parameters (protein:
+ * the rows of per-sequence protein sketches).
+ * A template is a KmerMinHash handle of which only num, ksize, is_protein, seed and max_hash are read (its
+ * content is neither read nor changed).  1 <= n_templates <= 6; each template has num > 0 or max_hash > 0,
+ * not both; DNA ksize 1 to 8192, protein ksize at least 3 (the per-object errors); seeds may differ and a
+ * template may appear twice (two equal collections).  A template that tracks abundance is refused:
+ * collections hold no abundances.  Input as smgpu_sketch_collection.  out has n_templates entries and
+ * receives collections the caller frees; on any error every out[m] is NULL. */
+void smgpu_sketch_collections(const char *buf /*[host|device]*/, const uint64_t *offsets /*[host|device], n_seqs + 1 */,
+                              uint64_t n_seqs, KmerMinHash *const *templates, uintptr_t n_templates, bool on_device,
+                              SketchCollection **out /* n_templates, caller frees each */);
 uint64_t smgpu_collection_len(SketchCollection *c);
 /* copy the packed rows to the host: hashes (capacity = the returned total) and offsets (n_rows + 1);
  * either may be NULL (call once with NULLs for the size) */
@@ -165,8 +183,9 @@ void smgpu_compare_path(int32_t path);
  * block whose hits overflow it (tests).  Results are identical. */
 void smgpu_find_path(int32_t path);
 /* Batch sketching of several k-sizes over the same sequences (smgpu_add_* with more than one
- * handle): on (default) = sketches with distinct k in {21, 31, 51} and one seed share a fused
- * launch that stages each tile of bases once; off = one launch per sketch.  Results are identical. */
+ * handle, smgpu_sketch_collections with more than one template): on (default) = sketches with
+ * distinct k in {21, 31, 51} and one seed share a fused launch that stages each tile of bases once;
+ * off = one launch per sketch or template.  Results are identical. */
 void smgpu_fuse_multi_k(bool on);
 /* LinearIndex::find (src/index/linear.rs:25-45) for every row of `queries` against `index`:
  * mode 0 = search_minhashes (node.similarity(query) > threshold), mode 1 =

@@ -102,6 +102,7 @@ EXTENSION_ABI = {
     "smgpu_collection_push_signatures": (None, [vp, vp, usz]),
     "smgpu_collection_from_csr": (vp, [vp, vp, u64, u32, u32, u64, u64, cb]),
     "smgpu_sketch_collection": (vp, [vp, vp, u64, u32, u32, u64, u64, cb]),
+    "smgpu_sketch_collections": (None, [vp, vp, u64, C.POINTER(vp), usz, cb, C.POINTER(vp)]),
     "smgpu_collection_len": (u64, [vp]),
     "smgpu_collection_copy": (u64, [vp, vp, vp]),
     "smgpu_collection_csr": (u64, [vp, C.POINTER(vp), C.POINTER(vp)]),
@@ -564,6 +565,22 @@ class SketchCollection:
             keep_o = np.ascontiguousarray(offsets, dtype=np.uint64)
             n_seqs = keep_o.size - 1
         return cls(_ptr=_call("smgpu_sketch_collection", _vp(keep_b), _vp(keep_o), n_seqs, num, ksize, seed, max_hash, on_device))
+
+    @classmethod
+    def sketch_sequences_multi(cls, buf, offsets, templates, on_device=False, n_seqs=None):
+        """One collection per template (a KmerMinHash whose parameters are used, not its content), each holding one
+        fresh sketch per sequence buf[offsets[s]:offsets[s+1]], all in one pass (smgpu_sketch_collections).
+        Returns the collections in template order."""
+        if on_device:
+            assert n_seqs is not None
+            keep_b, keep_o = buf, offsets
+        else:
+            keep_b = buf if isinstance(buf, (int, np.ndarray)) else bytes(buf)
+            keep_o = np.ascontiguousarray(offsets, dtype=np.uint64)
+            n_seqs = keep_o.size - 1
+        out = (vp * max(1, len(templates)))()
+        _call("smgpu_sketch_collections", _vp(keep_b), _vp(keep_o), n_seqs, _handles(templates), len(templates), on_device, out)
+        return [cls(_ptr=out[m]) for m in range(len(templates))]
 
     def rows_np(self):
         """The packed sketches as a list of numpy arrays (copies the CSR to the host)."""

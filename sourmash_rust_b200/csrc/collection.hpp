@@ -3,6 +3,7 @@
 // Replaces, for whole collections, the reference's Vec<Leaf<Signature>> walked pair by pair
 // (src/index/linear.rs:25-45, src/index.rs:131-160).
 #pragma once
+#include <memory>
 #include <vector>
 
 #include "minhash.hpp"
@@ -48,6 +49,9 @@ struct SketchCollection {
 // one fresh sketch per sequence of the batch, in one pass (sketch_many.cu); see include/sourmash_b200.h
 SketchCollection *sketch_collection(const uint8_t *buf, const uint64_t *offsets, uint64_t n_seqs, uint32_t num, uint32_t ksize,
                                     uint64_t seed, uint64_t max_hash, bool on_device);
+// the same for 1 to 6 parameter sets over one batch: one collection per entry of ps, in that order
+std::vector<std::unique_ptr<SketchCollection>> sketch_collections(const uint8_t *buf, const uint64_t *offsets, uint64_t n_seqs,
+                                                                  const std::vector<SketchParams> &ps, bool on_device);
 
 // see collection.cu: join_table_build
 struct JoinTable {

@@ -632,6 +632,32 @@ SketchCollection *smgpu_sketch_collection(const char *buf, const uint64_t *offse
                                                                               ksize, seed, max_hash, on_device));
     });
 }
+void smgpu_sketch_collections(const char *buf, const uint64_t *offsets, uint64_t n_seqs, KmerMinHash *const *templates,
+                              uintptr_t n_templates, bool on_device, SketchCollection **out) {
+    if (out)
+        for (uintptr_t m = 0; m < n_templates; m++) out[m] = nullptr;
+    landingpad_void([&]() {
+        nonnull(out, "out");
+        if (n_templates) nonnull(templates, "templates");
+        if (n_seqs) { nonnull(offsets, "offsets"); }
+        if (n_templates < 1 || n_templates > 6) smb200::throw_internal("sketch_collections takes 1 to 6 templates");
+        std::vector<smb200::SketchParams> ps(n_templates);
+        {
+            GuardN lk;
+            for (uintptr_t m = 0; m < n_templates; m++) lk.add(mh(templates[m])->mu);
+            lk.lock();
+            for (uintptr_t m = 0; m < n_templates; m++) {
+                const MH *t = mh(templates[m]);
+                if (t->track_abundance())
+                    smb200::throw_internal("a sketch collection holds no abundances: a template that tracks abundance is refused");
+                ps[m] = {t->num, t->ksize, t->is_protein, t->seed, t->max_hash};
+            }
+        }
+        std::vector<std::unique_ptr<COLL>> cs =
+            smb200::sketch_collections(reinterpret_cast<const uint8_t *>(buf), offsets, n_seqs, ps, on_device);
+        for (uintptr_t m = 0; m < n_templates; m++) out[m] = reinterpret_cast<SketchCollection *>(cs[m].release());
+    });
+}
 uint64_t smgpu_collection_len(SketchCollection *c) {
     return landingpad<uint64_t>([&]() { COLL *cc = coll(c); Guard lk(cc->mu); return cc->dirty ? (uint64_t)cc->h_nums.size() : cc->n_rows; });
 }

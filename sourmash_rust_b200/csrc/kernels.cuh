@@ -75,8 +75,20 @@ struct ProteinBatch {
 };
 uint64_t protein_slots(uint64_t n_bytes, uint64_t n_seqs);
 // aa, comp: protein_slots + 1 bytes; flags, pre: protein_slots + 1 u64; scan_tmp: scan_tmp_bytes(protein_slots + 1)
+// translate -> scan -> compact, then hash: launch_protein_translate + launch_protein_hash
 void launch_protein_sketch(const ProteinBatch &pb, const SketchOut &out, uint8_t *aa, uint8_t *comp, uint64_t *flags,
                            uint64_t *pre, void *scan_tmp, cudaStream_t st);
+// the residues of every sequence of at least pb.ksize bases, compacted into comp (pb.seed is not read);
+// pre[t] = kept residues before slot t
+void launch_protein_translate(const ProteinBatch &pb, uint8_t *aa, uint8_t *comp, uint64_t *flags, uint64_t *pre,
+                              void *scan_tmp, cudaStream_t st);
+// windows of pb.ksize / 3 residues of the sequences of at least pb.ksize bases, hashed with pb.seed; needs a translation
+// with a pb.ksize no larger than this one's.  Survivor positions are compacted residue indices.
+void launch_protein_hash(const ProteinBatch &pb, const SketchOut &out, const uint8_t *comp, const uint64_t *flags,
+                         const uint64_t *pre, cudaStream_t st);
+// starts[s] = compacted index of the first residue of sequence s (s <= n_seqs): pre at its slot region 2 offsets[s] + 6 s
+void launch_protein_seq_starts(const uint64_t *offsets, uint64_t n_seqs, const uint64_t *pre, uint64_t *starts,
+                               cudaStream_t st);
 
 // ---- sortops.cu -------------------------------------------------------------------------
 // keep[i] = hashes[i] passing the state-independent gate (h <= max_hash || max_hash == 0) and

@@ -676,6 +676,20 @@ struct PerSketch {
 };
 }  // namespace
 
+std::vector<int> fused_members(const std::vector<SketchParams> &ps) {
+    std::vector<int> fused;
+    if (!g_fuse_multi_k) return fused;
+    for (int i = 0; i < (int)ps.size(); i++) {
+        if (ps[i].is_protein || !sketch_has_fast_path(ps[i].ksize)) continue;
+        bool ok = fused.empty() || ps[fused[0]].seed == ps[i].seed;
+        for (int j : fused) ok = ok && ps[j].ksize != ps[i].ksize;
+        if (ok && fused.size() < 3) fused.push_back(i);
+    }
+    std::sort(fused.begin(), fused.end(), [&](int a, int b) { return ps[a].ksize < ps[b].ksize; });
+    if (fused.size() < 2) fused.clear();
+    return fused;
+}
+
 void KmerMinHash::add_sequences(KmerMinHash *const *mhs, int n_mhs, const SeqBatch &batch, bool force) {
     if (n_mhs <= 0) return;
     if (n_mhs > 6) throw_internal("at most 6 sketches per batch call");
@@ -816,18 +830,9 @@ void KmerMinHash::add_sequences(KmerMinHash *const *mhs, int n_mhs, const SeqBat
     }
     // DNA sketches with distinct fast-path k-sizes and one seed share a fused launch per chunk: the
     // tile is staged once and every k-size walks it (sketch.cu).  Member order = ascending k.
-    std::vector<int> fused;
-    if (g_fuse_multi_k) {
-        for (int i = 0; i < n_mhs; i++) {
-            const KmerMinHash &mh = *mhs[i];
-            if (mh.is_protein || !sketch_has_fast_path(mh.ksize)) continue;
-            bool ok = fused.empty() || mhs[fused[0]]->seed == mh.seed;
-            for (int j : fused) ok = ok && mhs[j]->ksize != mh.ksize;
-            if (ok && fused.size() < 3) fused.push_back(i);
-        }
-        std::sort(fused.begin(), fused.end(), [&](int a, int b) { return mhs[a]->ksize < mhs[b]->ksize; });
-        if (fused.size() < 2) fused.clear();
-    }
+    std::vector<SketchParams> params(n_mhs);
+    for (int i = 0; i < n_mhs; i++) params[i] = {mhs[i]->num, mhs[i]->ksize, mhs[i]->is_protein, mhs[i]->seed, mhs[i]->max_hash};
+    const std::vector<int> fused = fused_members(params);
     auto in_fused = [&](int i) { return std::find(fused.begin(), fused.end(), i) != fused.end(); };
     size_t ev_i = 0;
     unsigned fused_turn = 0;

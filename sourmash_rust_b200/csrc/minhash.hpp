@@ -23,6 +23,17 @@ extern bool g_fuse_multi_k;
 // host batches are copied to the device in chunks of this size, overlapped with the kernels (minhash.cu)
 extern uint64_t g_h2d_chunk_bytes;
 
+// what KmerMinHash::new takes apart from track_abundance
+struct SketchParams {
+    uint32_t num, ksize;
+    bool is_protein;
+    uint64_t seed, max_hash;
+};
+// Several sketches over one batch: those that share one fused launch (sketch.cu) -- with g_fuse_multi_k on, DNA
+// sketches of distinct fast-path k-sizes and the seed of the first of them, at most three -- in ascending k.
+// Empty unless at least two qualify.
+std::vector<int> fused_members(const std::vector<SketchParams> &ps);
+
 // A batch of sequences as the caller holds it (host or device memory).
 //   offsets == nullptr && read_len == 0 : one sequence of n_bytes
 //   offsets == nullptr && read_len  > 0 : n_seqs reads of read_len bytes, back to back

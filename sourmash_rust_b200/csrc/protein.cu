@@ -8,6 +8,9 @@
 // it frame f (order fw0, rc0, fw1, rc1, fw2, rc2 -- the order the reference adds them) owns
 // cap = len/3 + 1 slots, one per codon.  translate -> exclusive scan of the kept flags -> compaction
 // -> one thread per kept residue hashes the window that starts there if it fits in its frame.
+// The first three steps do not depend on the window size or the seed (beyond skipping sequences shorter
+// than pb.ksize), so several protein sketches of one batch can share them and run only the hash step
+// each; the hash step skips sequences shorter than its own pb.ksize.
 #include "device.hpp"
 #include "kernels.cuh"
 #include "murmur3.cuh"
@@ -100,7 +103,7 @@ __global__ void __launch_bounds__(256) protein_hash_kernel(const ProteinBatch pb
             const uint64_t f = (t - region) / cap;
             const uint64_t frame_end = pre[region + (f + 1) * cap];  // kept residues before the next frame
             p = pre[t];
-            if (p + aa_k <= frame_end) {
+            if (len >= pb.ksize && p + aa_k <= frame_end) {  // a sequence shorter than ksize adds nothing
                 h = murmur3_h1_bytes(comp + p, aa_k, pb.seed);
                 pass = h <= thr;
             }
@@ -123,18 +126,47 @@ __global__ void __launch_bounds__(256) protein_hash_kernel(const ProteinBatch pb
 
 uint64_t protein_slots(uint64_t n_bytes, uint64_t n_seqs) { return 2 * n_bytes + 6 * n_seqs; }
 
-void launch_protein_sketch(const ProteinBatch &pb, const SketchOut &out, uint8_t *aa, uint8_t *comp, uint64_t *flags,
-                           uint64_t *pre, void *scan_tmp, cudaStream_t st) {
+static unsigned protein_blocks(uint64_t total) {
+    const uint64_t b = (total + 255) / 256;
+    return (unsigned)(b > 148 * 32 ? 148 * 32 : b);
+}
+
+void launch_protein_translate(const ProteinBatch &pb, uint8_t *aa, uint8_t *comp, uint64_t *flags, uint64_t *pre,
+                              void *scan_tmp, cudaStream_t st) {
     const uint64_t total = protein_slots(pb.n, pb.n_seqs);
     if (!total) return;
-    uint64_t b = (total + 255) / 256;
-    const unsigned blocks = (unsigned)(b > 148 * 32 ? 148 * 32 : b);
+    const unsigned blocks = protein_blocks(total);
     protein_translate_kernel<<<blocks, 256, 0, st>>>(pb, total, aa, flags);
     SM_LAUNCHED();
     scan_exclusive_u64(flags, pre, total + 1, scan_tmp, st);
     protein_compact_kernel<<<blocks, 256, 0, st>>>(aa, flags, pre, total, comp);
     SM_LAUNCHED();
-    protein_hash_kernel<<<blocks, 256, 0, st>>>(pb, total, flags, pre, comp, out);
+}
+
+void launch_protein_hash(const ProteinBatch &pb, const SketchOut &out, const uint8_t *comp, const uint64_t *flags,
+                         const uint64_t *pre, cudaStream_t st) {
+    const uint64_t total = protein_slots(pb.n, pb.n_seqs);
+    if (!total) return;
+    protein_hash_kernel<<<protein_blocks(total), 256, 0, st>>>(pb, total, flags, pre, comp, out);
+    SM_LAUNCHED();
+}
+
+void launch_protein_sketch(const ProteinBatch &pb, const SketchOut &out, uint8_t *aa, uint8_t *comp, uint64_t *flags,
+                           uint64_t *pre, void *scan_tmp, cudaStream_t st) {
+    launch_protein_translate(pb, aa, comp, flags, pre, scan_tmp, st);
+    launch_protein_hash(pb, out, comp, flags, pre, st);
+}
+
+__global__ void __launch_bounds__(256) protein_seq_starts_kernel(const uint64_t *__restrict__ offsets, uint64_t n_seqs,
+                                                                 const uint64_t *__restrict__ pre, uint64_t *starts) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t s = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; s <= n_seqs; s += stride)
+        starts[s] = pre[2 * offsets[s] + 6 * s];
+}
+
+void launch_protein_seq_starts(const uint64_t *offsets, uint64_t n_seqs, const uint64_t *pre, uint64_t *starts,
+                               cudaStream_t st) {
+    protein_seq_starts_kernel<<<protein_blocks(n_seqs + 1), 256, 0, st>>>(offsets, n_seqs, pre, starts);
     SM_LAUNCHED();
 }
 
