@@ -150,6 +150,18 @@ KB_HD void extract2w(const uint32_t *w, uint32_t s, uint32_t (&e)[KmerGeom<K>::N
     e[KmerGeom<K>::NE - 1] &= KmerGeom<K>::TOP2;
 }
 
+// N words of a stream starting at bit s of w[0] (reads w[0 .. N]; only the low 5 bits of `s` are used)
+template <int N>
+KB_HD void funnel_words(const uint32_t *w, uint32_t s, uint32_t (&e)[N]) {
+    uint32_t prev = w[0];
+#pragma unroll
+    for (int j = 0; j < N; j++) {
+        const uint32_t next = w[j + 1];
+        e[j] = kb_funnel_r(prev, next, s);
+        prev = next;
+    }
+}
+
 // NE words whose TOP bits are the k-mer's last base: `w`/`s` address bit 2 * (start + K) - 32 * NE of
 // the stream, so the 32 * NE - 2K low bits are whatever precedes the k-mer.  For ODD K that is
 // harmless to canonical_is_fw: a k-mer of odd length never equals its reverse complement, so the
@@ -158,14 +170,41 @@ KB_HD void extract2w(const uint32_t *w, uint32_t s, uint32_t (&e)[KmerGeom<K>::N
 template <int K>
 KB_HD void extract2_end(const uint32_t *w, uint32_t s, uint32_t (&e)[KmerGeom<K>::NE]) {
     static_assert(K % 2 == 1, "end-aligned strand comparison needs an odd k");
-    uint32_t prev = w[0];
-#pragma unroll
-    for (int j = 0; j < KmerGeom<K>::NE; j++) {
-        const uint32_t next = w[j + 1];
-        e[j] = kb_funnel_r(prev, next, s);
-        prev = next;
-    }
+    funnel_words<KmerGeom<K>::NE>(w, s, e);
 }
+
+KB_HD constexpr int kb_max3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
+
+// End-aligned 2-bit words of every k-size of a fused launch (KB / KC = 0: absent) from ONE extraction per strand.
+//   reverse complement: rc(window i) of every k-size ends at base B - i of the rc stream, so extract2_end<K> there
+//     is the top NE(K) of the NR = NE(KM) words extract2_end<KM> takes -- whole words, no shift;
+//   forward: window i of k-size K ends at base i + K, a different place per k-size.  NF words ending at base i + KM
+//     reach back far enough to hold every k-size's end-aligned words, which then sit at a constant bit offset
+//     (fw_bit<K>): one funnel shift per word where that offset is not a multiple of 32.
+// F is funnel_words<NF> at base i + KM - 16 * NF of the forward stream, R is extract2_end<KM> of the rc stream.
+template <int KA, int KB, int KC>
+struct FusedGeom {
+    static constexpr int KM = kb_max3(KA, KB, KC);
+    KB_HD static constexpr int lo(int K) { return K ? K - 16 * ((2 * K + 31) / 32) : 0; }  // first base of extract2_end<K>, from i
+    static constexpr int LO = lo(KA) < lo(KB) ? (lo(KA) < lo(KC) ? lo(KA) : lo(KC)) : (lo(KB) < lo(KC) ? lo(KB) : lo(KC));
+    static constexpr int NF = (KM - LO + 15) / 16;
+    static constexpr int NR = KmerGeom<KM>::NE;
+    template <int K>
+    KB_HD static constexpr int fw_bit() { return 2 * (lo(K) - (KM - 16 * NF)); }
+
+    template <int K>
+    KB_HD static void split(const uint32_t (&F)[NF], const uint32_t (&R)[NR], uint32_t (&ef)[KmerGeom<K>::NE],
+                            uint32_t (&er)[KmerGeom<K>::NE]) {
+        constexpr int NE = KmerGeom<K>::NE, W = fw_bit<K>() / 32, S = fw_bit<K>() % 32;
+        static_assert(K % 2 == 1 && K <= KM && fw_bit<K>() >= 0 && W + NE + (S != 0) <= NF, "fused strand geometry");
+#pragma unroll
+        for (int j = 0; j < NE; j++) {
+            if constexpr (S != 0) ef[j] = kb_funnel_r(F[W + j], F[W + j + 1], (uint32_t)S);
+            else ef[j] = F[W + j];
+            er[j] = R[NR - NE + j];
+        }
+    }
+};
 
 // lexicographic `fw < rc` (src/lib.rs:263) from the little-endian 2-bit integers of the two
 // strands: with comp(c) = ~c, BE(fw) = ~E(rc) and BE(rc) = ~E(fw), so fw <lex rc <=> E(fw) < E(rc).
@@ -263,6 +302,31 @@ KB_HD uint32_t dilate_word(uint32_t in0, uint32_t in1, uint32_t in2, int span) {
         d0 |= y0;
     }
     return d0;
+}
+
+KB_HD constexpr int kb_floor_pow2(int x) { return x < 2 ? 1 : 2 * kb_floor_pow2(x / 2); }
+
+// out[j] = dilate_word(in0, in1, in2, K_j - d) for every k-size K_j of {KA, KB, KC} that is not 0, d = 0 or 1, from
+// ONE doubling chain: D_1, D_2, D_4, ... is the same for every span, and span K - d takes D_a for the largest power of
+// two a <= K (the same a for K and K - 1, as K is not a power of two) and one last shift by K - d - a < a <= 32.
+template <int KA, int KB, int KC>
+KB_HD void dilate_words(uint32_t in0, uint32_t in1, uint32_t in2, uint32_t d, uint32_t (&out)[3]) {
+    constexpr int KM = kb_max3(KA, KB, KC);
+    static_assert(KM <= 64, "spans up to 64");
+    static_assert((KA > 2 && KA != kb_floor_pow2(KA)) && (!KB || (KB > 2 && KB != kb_floor_pow2(KB))) &&
+                      (!KC || (KC > 2 && KC != kb_floor_pow2(KC))),
+                  "K and K - 1 must share their power-of-two step");
+    uint32_t d0 = in0, d1 = in1, d2 = in2;
+#pragma unroll
+    for (int a = 1; a <= 32; a *= 2) {
+        if (KA && kb_floor_pow2(KA) == a) out[0] = d0 | kb_funnel_r(d0, d1, (uint32_t)(KA - a) - d);
+        if (KB && kb_floor_pow2(KB) == a) out[1] = d0 | kb_funnel_r(d0, d1, (uint32_t)(KB - a) - d);
+        if (KC && kb_floor_pow2(KC) == a) out[2] = d0 | kb_funnel_r(d0, d1, (uint32_t)(KC - a) - d);
+        if (2 * a > KM) break;
+        uint32_t y0 = d0, y1 = d1, y2 = d2;
+        kb_shr96(y0, y1, y2, a);
+        d0 |= y0; d1 |= y1; d2 |= y2;
+    }
 }
 
 }  // namespace smb200

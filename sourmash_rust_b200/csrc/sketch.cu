@@ -18,7 +18,8 @@
 //     bitmap; a second short phase dilates the invalid/sequence-end bitmaps into a
 //     "window start is unusable" bitmap per k-size;
 //   * one launch serves up to three sketches (k-sizes) of the same batch: the staging above is
-//     done once per tile, then one k-mer loop per k-size walks it;
+//     done once per tile, then one fused k-mer loop walks it, each trip handling one window start
+//     for every k-size (shared 2-bit extractions and validity load);
 //   * one thread per k-mer: one bit test for validity, two unaligned end-aligned 2-bit extractions
 //     + one integer compare for the canonical strand, one unaligned ASCII extraction of the
 //     chosen strand, MurmurHash3 x64_128 fully unrolled for the compile-time K (murmur3.cuh),
@@ -90,8 +91,11 @@ struct TileViews {
     uint32_t *r2;     // SK_PAD2 + B/16 + 2 words
     uint32_t *bad;    // B/32 + 3 words   invalid-base bitmap
     uint32_t *end;    // B/32 + 3 words   "last base of a sequence" bitmap
-    uint32_t *sbad;   // nk * TILE/32 words   window start unusable, one bitmap per k-size of the launch
+    uint32_t *sbad;   // sbad_stride(nk) * TILE/32 words, 16-byte aligned: window start unusable, one bitmap per k-size of
+                      // the launch, interleaved -- word w of k-size j at sbad[w * sbad_stride(nk) + j]
 };
+// words per 32 window starts in sbad: the words of all k-sizes of a launch are one 32-, 64- or 128-bit load
+__host__ __device__ constexpr int sbad_stride(int nk) { return nk == 3 ? 4 : nk; }
 constexpr int SK_PAD2 = 4;  // words in front of each 2-bit stream (extract2_end reaches up to 64 bases back)
 __host__ __device__ constexpr int tile_bases(int K) { return SK_TILE + ((K - 1 + 15) / 16) * 16; }
 // words between the byte-shifted copies of an ASCII strand: at least the (B + 8) bytes of one copy, and
@@ -106,8 +110,8 @@ __host__ __device__ constexpr size_t tile_smem_bytes(int B, int nk = 1) {
            + (SK_SHIFTED ? 8 * (size_t)copy_stride_words(B) * 4 : 2 * ((size_t)B + 16))   // fA, rA (+ their byte-shifted copies)
            + 2 * ((size_t)B / 4 + 8 + 4 * SK_PAD2)  // f2, r2
            + 2 * ((size_t)(B + 31) / 32 * 4 + 12)  // bad, end
-           + (size_t)nk * (SK_TILE / 8)   // sbad
-           + 128;                         // alignment slack
+           + (size_t)sbad_stride(nk) * (SK_TILE / 8)   // sbad
+           + 128;                         // alignment slack (sbad's 16-byte alignment)
 }
 __device__ __forceinline__ TileViews carve_tile(uint8_t *base, int B) {
     TileViews v;
@@ -121,7 +125,7 @@ __device__ __forceinline__ TileViews carve_tile(uint8_t *base, int B) {
     const int wm = (B + 31) / 32 + 3;
     v.bad = reinterpret_cast<uint32_t *>(p); p += wm * 4;
     v.end = reinterpret_cast<uint32_t *>(p); p += wm * 4;
-    v.sbad = reinterpret_cast<uint32_t *>(p);
+    v.sbad = reinterpret_cast<uint32_t *>(base + ((p - base + 15) & ~15));
     return v;
 }
 
@@ -260,6 +264,44 @@ __device__ __forceinline__ void build_start_bitmap(const TileViews &v, uint32_t 
     }
 }
 
+// build_start_bitmap for every k-size of a fused launch (two or three), interleaved (sbad_stride), in one pass over all
+// threads: the two lanes of a pair take the same word w, the even one dilates `bad` over K, the odd one `end` over
+// K - 1, each with one doubling chain for all k-sizes (dilate_words); the even lane combines the two, stores the
+// words and reports first_bad.  (The single-k kernels keep build_start_bitmap: with one span there is no chain to
+// share, and the pairs measured 0.02 ms per launch slower there, profiles/sketch_pipes_r4.md.)
+template <int KA, int KB, int KC>
+__device__ __forceinline__ void build_start_bitmaps(const TileViews &v, uint64_t t0, const SketchBatch &sb,
+                                                    const SketchOuts &outs) {
+    constexpr int NK = KC ? 3 : 2, NKP = sbad_stride(NK);
+    static_assert(KB != 0 && (2 * (SK_TILE / 32)) % 32 == 0 && SK_THREADS % 32 == 0, "whole warps take part in the shuffle");
+    for (int t = threadIdx.x; t < 2 * (SK_TILE / 32); t += blockDim.x) {
+        const int w = t >> 1;
+        const uint32_t odd = (uint32_t)t & 1u;
+        const uint32_t *src = (odd ? v.end : v.bad) + w;
+        uint32_t d[3], o[3];
+        dilate_words<KA, KB, KC>(src[0], src[1], src[2], odd, d);  // even lane: hasbad, odd lane: crosses
+#pragma unroll
+        for (int j = 0; j < NK; j++) o[j] = __shfl_xor_sync(0xFFFFFFFFu, d[j], 1);
+        if (!odd) {
+            // starts at or beyond the limit / the buffer are never used
+            const uint64_t q0 = t0 + (uint64_t)w * 32;
+            uint32_t beyond = 0;
+            if (q0 + 32 > sb.n_limit) beyond = (q0 >= sb.n_limit) ? 0xFFFFFFFFu : (0xFFFFFFFFu << (uint32_t)(sb.n_limit - q0));
+            uint32_t s[4] = {0, 0, 0, 0};
+#pragma unroll
+            for (int j = 0; j < NK; j++) {
+                s[j] = d[j] | o[j] | beyond;
+                const uint32_t err = d[j] & ~o[j] & ~beyond;
+                if (err && outs.first_bad[j])
+                    atomicMin(outs.first_bad[j], (unsigned long long)(sb.pos_base + q0 + (uint32_t)(__ffs(err) - 1)));
+            }
+            uint32_t *dst = v.sbad + w * NKP;
+            if constexpr (NKP == 4) *reinterpret_cast<uint4 *>(dst) = make_uint4(s[0], s[1], s[2], s[3]);
+            else *reinterpret_cast<uint2 *>(dst) = make_uint2(s[0], s[1]);
+        }
+    }
+}
+
 // Survivors are rare (1 window in 1000 for scaled=1000), so the common path is one predicated
 // branch; the threads that do pass aggregate their slot request over whoever is in the branch
 // with them (a num sketch that is still filling passes every window: one atomic per warp then).
@@ -287,6 +329,45 @@ __device__ __forceinline__ void append_survivor(bool pass, uint64_t h, uint64_t 
 // ---------------------------------------------------------------------------------------
 // fast path: compile-time k-sizes; one launch serves up to three sketches of the same batch
 // ---------------------------------------------------------------------------------------
+// Prefilter on the high words.  The hash is xs(a) + xs(b) (murmur3_h1_words_parts) and xs keeps the high word, so its
+// high word is hi(a) + hi(b) + carry, carry 0 or 1: h <= thr needs s = hi(a) + hi(b) (mod 2^32) in [0, hi(thr)] or
+// s = 2^32 - 1, i.e. s + 1 <= hi(thr) + 1 (mod 2^32; every s when hi(thr) = 2^32 - 1).  Only the windows that pass
+// finish the hash (two xorshifts, a 64-bit add and compare) and test h <= thr exactly.
+__device__ __forceinline__ uint32_t prefilter_limit(uint64_t thr) {
+    const uint32_t thr_hi = (uint32_t)(thr >> 32);
+    uint32_t lim = thr_hi == 0xFFFFFFFFu ? thr_hi : thr_hi + 1u;
+    asm("" : "+r"(lim));  // opaque: computed once, not again per window
+    return lim;
+}
+
+// One window of k-size K after its 2-bit words are extracted: strand choice, the ASCII words of the chosen strand
+// (pf / pr: the window's words on the forward / rc strand; sf / sr: their byte shifts when SK_SHIFTED is off),
+// MurmurHash3, the prefilter and the survivor append.
+template <int K>
+__device__ __forceinline__ void kmer_window(const uint32_t (&ef)[KmerGeom<K>::NE], const uint32_t (&er)[KmerGeom<K>::NE],
+                                            bool valid, const uint32_t *pf, const uint32_t *pr, uint32_t sf, uint32_t sr,
+                                            uint32_t lim, uint64_t thr, uint64_t pos0, const SketchBatch &sb,
+                                            const SketchOut &out) {
+    using G = KmerGeom<K>;
+    const bool use_fw = canonical_is_fw<K>(ef, er);
+    uint32_t kw[G::NW];
+    const uint32_t *pa = use_fw ? pf : pr;
+#if SK_SHIFTED
+    (void)sf; (void)sr;
+#pragma unroll
+    for (int j = 0; j < G::NW; j++) kw[j] = pa[j];
+    kw[G::NW - 1] &= G::TOPA;
+#else
+    extractAw<K>(pa, use_fw ? sf : sr, kw);
+#endif
+    uint64_t a, b;
+    murmur3_h1_words_parts<K>(kw, sb.seed, a, b);
+    if (valid & ((uint32_t)(a >> 32) + (uint32_t)(b >> 32) + 1u <= lim)) {  // `&`: one test, no early branch
+        const uint64_t h = mm_xorshift33(a) + mm_xorshift33(b);
+        append_survivor(h <= thr, h, pos0, sb, out);
+    }
+}
+
 // The k-mer loop of one k-size over a staged tile of B bases: one thread per window start
 // i = r * SK_THREADS + tid.  Per-thread constants:
 //   2-bit views: word (i >> 4), bit shift 2 * (i & 15); rc(window i) starts at base B - K - i of the
@@ -308,6 +389,7 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
 #if SK_SHIFTED
     constexpr int CS = copy_stride_words(B);  // words between the byte-shifted copies of a strand
     const uint32_t *qfa = v.fA + (tid & 3) * CS + (tid >> 2), *qra = v.rA + (ri0 & 3) * CS + (ri0 >> 2);
+    const uint32_t sfa = 0, sra = 0;
     (void)ra0;
 #else
     const uint32_t *qfa = v.fA + (tid >> 2), *qra = v.fA + (ra0 >> 2);
@@ -317,13 +399,7 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
     const uint32_t *qsb = sbad + (tid >> 5);
     uint32_t mb = 1u << (tid & 31);
     asm("" : "+r"(mb));  // opaque: keeps the validity test a single LOP3 against a resident mask
-    // Prefilter on the high words.  The hash is xs(a) + xs(b) (murmur3_h1_words_parts) and xs keeps the high word, so
-    // its high word is hi(a) + hi(b) + carry, carry 0 or 1: h <= thr needs s = hi(a) + hi(b) (mod 2^32) in
-    // [0, hi(thr)] or s = 2^32 - 1, i.e. s + 1 <= hi(thr) + 1 (mod 2^32; every s when hi(thr) = 2^32 - 1).  Only the
-    // windows that pass finish the hash (two xorshifts, a 64-bit add and compare) and test h <= thr exactly.
-    const uint32_t thr_hi = (uint32_t)(thr >> 32);
-    uint32_t lim = thr_hi == 0xFFFFFFFFu ? thr_hi : thr_hi + 1u;
-    asm("" : "+r"(lim));  // opaque: computed once, not again per window
+    const uint32_t lim = prefilter_limit(thr);
     // running word pointers: stepped once per UNROLL windows, constant offsets inside
 #pragma unroll 1
     for (int r = 0; r < SK_TILE / SK_THREADS; r += UNROLL) {
@@ -333,22 +409,8 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
             uint32_t ef[G::NE], er[G::NE];
             extract2_end<K>(qf2 + u * (SK_THREADS / 16), sf2, ef);
             extract2_end<K>(qr2 - u * (SK_THREADS / 16), sr2, er);  // rc(window i) starts at B - K - i
-            const bool use_fw = canonical_is_fw<K>(ef, er);
-            uint32_t kw[G::NW];
-            const uint32_t *pa = use_fw ? qfa + u * (SK_THREADS / 4) : qra - u * (SK_THREADS / 4);
-#if SK_SHIFTED
-#pragma unroll
-            for (int j = 0; j < G::NW; j++) kw[j] = pa[j];
-            kw[G::NW - 1] &= G::TOPA;
-#else
-            extractAw<K>(pa, use_fw ? sfa : sra, kw);
-#endif
-            uint64_t a, b;
-            murmur3_h1_words_parts<K>(kw, sb.seed, a, b);
-            if (valid & ((uint32_t)(a >> 32) + (uint32_t)(b >> 32) + 1u <= lim)) {  // `&`: one test, no early branch
-                const uint64_t h = mm_xorshift33(a) + mm_xorshift33(b);
-                append_survivor(h <= thr, h, t0 + (uint32_t)((r + u) * SK_THREADS), sb, out);
-            }
+            kmer_window<K>(ef, er, valid, qfa + u * (SK_THREADS / 4), qra - u * (SK_THREADS / 4), sfa, sra, lim, thr,
+                           t0 + (uint32_t)((r + u) * SK_THREADS), sb, out);
         }
         qf2 += UNROLL * (SK_THREADS / 16); qr2 -= UNROLL * (SK_THREADS / 16);
         qfa += UNROLL * (SK_THREADS / 4);  qra -= UNROLL * (SK_THREADS / 4);
@@ -356,7 +418,103 @@ __device__ __forceinline__ void kmer_loop(const TileViews &v, const uint32_t *sb
     }
 }
 
-__host__ __device__ constexpr int kmax3(int a, int b, int c) { return a > b ? (a > c ? a : c) : (b > c ? b : c); }
+// The k-mer loop of a fused launch (two or three k-sizes; KC = 0: absent): one trip handles window start
+// i = r * SK_THREADS + tid for every k-size.  What is the same for all of them is done once per window start:
+//   * one forward and one reverse-complement 2-bit extraction, from which every k-size takes its end-aligned words
+//     (FusedGeom: the rc words are shared as they are, the forward ones at a constant shift);
+//   * one 64- or 128-bit load of the interleaved validity words (sbad_stride);
+//   * the forward ASCII pointer (a window's forward bytes start at byte i for every k-size), and one rc ASCII pointer
+//     per K mod 4: rc(window i) starts at byte B - K - i, so k-sizes with equal K mod 4 read the same byte-shifted
+//     copy, (K' - K) / 4 words apart;
+//   * one trip counter and one set of running pointers.
+template <int KA, int KB, int KC, int B, int UNROLL>
+__device__ __forceinline__ void kmer_loop_fused(const TileViews &v, const uint64_t (&thr)[3], const uint64_t t0,
+                                                const SketchBatch &sb, const SketchOuts &outs) {
+    using FG = FusedGeom<KA, KB, KC>;
+    constexpr int NK = KC ? 3 : 2, NKP = sbad_stride(NK);
+    constexpr int Ks[3] = {KA, KB, KC};
+    // rc ASCII pointer of k-size j: that of root[j], the first k-size with the same K mod 4, minus (K_j - K_root) / 4 words
+    constexpr int root[3] = {0, (KB - KA) % 4 ? 1 : 0, (KC - KA) % 4 == 0 ? 0 : (KC - KB) % 4 == 0 ? 1 : 2};
+    static_assert(KB != 0 && SK_THREADS % 32 == 0 && 16 * FG::NF - FG::KM <= 16 * SK_PAD2, "k-mer loop addressing");
+    const int tid = threadIdx.x;
+    const int ef0 = tid + FG::KM - 16 * FG::NF, er0 = B - tid - 16 * FG::NR;  // >= -16 * SK_PAD2
+    const uint32_t *qf2 = v.f2 + (ef0 >> 4), *qr2 = v.r2 + (er0 >> 4);  // arithmetic shifts: floor
+    const uint32_t sf2 = (uint32_t)ef0 * 2u, sr2 = (uint32_t)er0 * 2u;  // funnel shifts use the low 5 bits
+    const uint32_t *qra[3];
+    uint32_t sra[3];
+#if SK_SHIFTED
+    constexpr int CS = copy_stride_words(B);
+    const uint32_t *qfa = v.fA + (tid & 3) * CS + (tid >> 2);
+    const uint32_t sfa = 0;
+#pragma unroll
+    for (int j = 0; j < NK; j++) {
+        const int ri0 = B - Ks[j] - tid;
+        qra[j] = root[j] == j ? v.rA + (ri0 & 3) * CS + (ri0 >> 2) : nullptr;
+        sra[j] = 0;
+    }
+#else
+    const uint32_t *qfa = v.fA + (tid >> 2);
+    const uint32_t sfa = (uint32_t)tid * 8u;
+#pragma unroll
+    for (int j = 0; j < NK; j++) {
+        const int ra0 = 2 * B + 16 - Ks[j] - tid;
+        qra[j] = root[j] == j ? v.fA + (ra0 >> 2) : nullptr;
+        sra[j] = (uint32_t)ra0 * 8u;
+    }
+#endif
+    const uint32_t *qsb = v.sbad + (tid >> 5) * NKP;
+    uint32_t mb = 1u << (tid & 31);
+    asm("" : "+r"(mb));  // opaque: keeps each validity test a single LOP3 against a resident mask
+    uint32_t lim[3];
+#pragma unroll
+    for (int j = 0; j < NK; j++) lim[j] = prefilter_limit(thr[j]);
+#pragma unroll 1
+    for (int r = 0; r < SK_TILE / SK_THREADS; r += UNROLL) {
+#pragma unroll
+        for (int u = 0; u < UNROLL; u++) {
+            uint32_t bad[4];
+            const uint32_t *pb = qsb + u * (SK_THREADS / 32) * NKP;
+            if constexpr (NKP == 4) {
+                const uint4 x = *reinterpret_cast<const uint4 *>(pb);
+                bad[0] = x.x; bad[1] = x.y; bad[2] = x.z; bad[3] = x.w;
+            } else {
+                const uint2 x = *reinterpret_cast<const uint2 *>(pb);
+                bad[0] = x.x; bad[1] = x.y;
+            }
+            uint32_t F[FG::NF], R[FG::NR];
+            funnel_words<FG::NF>(qf2 + u * (SK_THREADS / 16), sf2, F);
+            funnel_words<FG::NR>(qr2 - u * (SK_THREADS / 16), sr2, R);
+            const uint64_t pos0 = t0 + (uint32_t)((r + u) * SK_THREADS);
+            const uint32_t *pf = qfa + u * (SK_THREADS / 4);
+            {
+                uint32_t ef[KmerGeom<KA>::NE], er[KmerGeom<KA>::NE];
+                FG::template split<KA>(F, R, ef, er);
+                kmer_window<KA>(ef, er, (bad[0] & mb) == 0, pf, qra[0] - u * (SK_THREADS / 4), sfa, sra[0], lim[0],
+                                thr[0], pos0, sb, outs.o[0]);
+            }
+            {
+                constexpr int K = KB, J = root[1];
+                uint32_t ef[KmerGeom<K>::NE], er[KmerGeom<K>::NE];
+                FG::template split<K>(F, R, ef, er);
+                kmer_window<K>(ef, er, (bad[1] & mb) == 0, pf, qra[J] - (K - Ks[J]) / 4 - u * (SK_THREADS / 4), sfa,
+                               sra[J], lim[1], thr[1], pos0, sb, outs.o[1]);
+            }
+            if constexpr (KC != 0) {
+                constexpr int K = KC, J = root[2];
+                uint32_t ef[KmerGeom<K>::NE], er[KmerGeom<K>::NE];
+                FG::template split<K>(F, R, ef, er);
+                kmer_window<K>(ef, er, (bad[2] & mb) == 0, pf, qra[J] - (K - Ks[J]) / 4 - u * (SK_THREADS / 4), sfa,
+                               sra[J], lim[2], thr[2], pos0, sb, outs.o[2]);
+            }
+        }
+        qf2 += UNROLL * (SK_THREADS / 16); qr2 -= UNROLL * (SK_THREADS / 16);
+        qfa += UNROLL * (SK_THREADS / 4);
+#pragma unroll
+        for (int j = 0; j < NK; j++)
+            if (root[j] == j) qra[j] -= UNROLL * (SK_THREADS / 4);
+        qsb += UNROLL * (SK_THREADS / 32) * NKP;
+    }
+}
 
 // KB / KC = 0: absent.  The tile (TMA copy, five views, sequence-end bitmap) is staged ONCE and every
 // k-size walks it: a multi-k batch (BASELINE cfg2: k = 21, 31, 51 over the same reads) reads each
@@ -364,14 +522,12 @@ __host__ __device__ constexpr int kmax3(int a, int b, int c) { return a > b ? (a
 template <int KA, int KB, int KC>
 __global__ void __launch_bounds__(SK_THREADS, SK_MIN_CTAS) sketch_kernel(const SketchBatch sb, const SketchOuts outs,
                                                                          uint32_t n_tiles) {
-    constexpr int B = tile_bases(kmax3(KA, KB, KC));
+    constexpr int B = tile_bases(kb_max3(KA, KB, KC));
     extern __shared__ __align__(128) uint8_t s_dyn[];
     __shared__ __align__(8) uint64_t s_bar;
     const TileViews v = carve_tile(s_dyn, B);
     const int tid = threadIdx.x;
-    const uint64_t thrA = *outs.o[0].thr;
-    const uint64_t thrB = KB ? *outs.o[1].thr : 0;
-    const uint64_t thrC = KC ? *outs.o[2].thr : 0;
+    const uint64_t thr[3] = {*outs.o[0].thr, KB ? *outs.o[1].thr : 0, KC ? *outs.o[2].thr : 0};
 
     // Tiles are handed out dynamically: a CTA's first tile is its block index, every further one
     // comes from an atomic counter.  (With a static round-robin the warp scheduler's fixed priority
@@ -415,16 +571,13 @@ __global__ void __launch_bounds__(SK_THREADS, SK_MIN_CTAS) sketch_kernel(const S
         build_shifted_copies(v, B);
 #endif
         __syncthreads();
-        build_start_bitmap(v, v.sbad, KA, t0, sb, outs.first_bad[0]);
-        if (KB) build_start_bitmap(v, v.sbad + SK_TILE / 32, KB, t0, sb, outs.first_bad[1]);
-        if (KC) build_start_bitmap(v, v.sbad + 2 * (SK_TILE / 32), KC, t0, sb, outs.first_bad[2]);
+        if constexpr (KB != 0) build_start_bitmaps<KA, KB, KC>(v, t0, sb, outs);
+        else build_start_bitmap(v, v.sbad, KA, t0, sb, outs.first_bad[0]);
         __syncthreads();
-        // (the fused forms unroll less: three loops unrolled by four no longer fit the instruction cache --
-        // ncu showed 11 % `no instruction` stalls)
-        constexpr int U = KB ? SK_UNROLL_FUSED : SK_UNROLL;
-        kmer_loop<KA, B, U>(v, v.sbad, thrA, t0, sb, outs.o[0]);
-        if (KB) kmer_loop<(KB ? KB : KA), B, U>(v, v.sbad + SK_TILE / 32, thrB, t0, sb, outs.o[1]);
-        if (KC) kmer_loop<(KC ? KC : KA), B, U>(v, v.sbad + 2 * (SK_TILE / 32), thrC, t0, sb, outs.o[2]);
+        // (the fused loop unrolls less: its body holds two or three hashes per window start, and a larger body no
+        // longer fits the instruction cache -- ncu showed 11 % `no instruction` stalls at three loops unrolled by four)
+        if constexpr (KB != 0) kmer_loop_fused<KA, KB, KC, B, SK_UNROLL_FUSED>(v, thr, t0, sb, outs);
+        else kmer_loop<KA, B, SK_UNROLL>(v, v.sbad, thr[0], t0, sb, outs.o[0]);
         if (tid == 0) s_next = after_next;
         __syncthreads();  // views are rebuilt by the next tile
         tile = next;
@@ -502,7 +655,7 @@ bool sketch_multi_supported(const uint32_t *ks, int nk) {
 template <int KA, int KB, int KC>
 static void launch_fast(const SketchBatch &sb, const SketchOuts &outs, uint32_t n_tiles, unsigned grid, cudaStream_t st) {
     constexpr int NK = 1 + (KB ? 1 : 0) + (KC ? 1 : 0);
-    constexpr size_t smem = tile_smem_bytes(tile_bases(kmax3(KA, KB, KC)), NK);
+    constexpr size_t smem = tile_smem_bytes(tile_bases(kb_max3(KA, KB, KC)), NK);
     static bool attr_set = false;
     if (!attr_set) {
         SM_CUDA(cudaFuncSetAttribute(sketch_kernel<KA, KB, KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
