@@ -270,7 +270,9 @@ uint64_t smgpu_nodegraph_unique_kmers(Nodegraph *ng);
  * Internal nodes compare as sbt.rs:233-277 (matches / min_n_below, matches / |query|), leaves as
  * index.rs:131-160.  hit_offsets (n_queries + 1, host) / hits (host, capacity hits_cap) receive, per
  * query, the POSITIONS of the matching leaves in the order the reference's depth-first walk
- * reaches them.  Returns the total number of hits. */
+ * reaches them.  Returns the total number of hits, of which the first hits_cap are written: a call
+ * with hits = NULL gives the total and the offsets.  At most 65535 internal nodes: with more, a call
+ * that has at least one query records an Internal error. */
 uint64_t smgpu_sbt_find(uint32_t d, const uint64_t *node_positions, Nodegraph *const *nodes, const uint64_t *min_n_below,
                         uint64_t n_nodes, const uint64_t *leaf_positions, SketchCollection *leaves,
                         SketchCollection *queries, int32_t mode, double threshold, uint64_t *hit_offsets, uint64_t *hits,

@@ -794,6 +794,26 @@ size_t orc_ng_get(const OrcNodegraph *ng, uint64_t hash) {
     }
     return 1;
 }
+/* count / get over a batch in one call: is_new[i] = count(hashes[i]) in batch order, present[i] = get(hashes[i]);
+ * either output may be NULL.  Return the sums. */
+uint64_t orc_ng_count_many(OrcNodegraph *ng, const uint64_t *hashes, size_t n, uint8_t *is_new) {
+    uint64_t sum = 0;
+    for (size_t i = 0; i < n; i++) {
+        const int v = orc_ng_count(ng, hashes[i]);
+        if (is_new) is_new[i] = (uint8_t)v;
+        sum += (uint64_t)v;
+    }
+    return sum;
+}
+uint64_t orc_ng_get_many(const OrcNodegraph *ng, const uint64_t *hashes, size_t n, uint8_t *present) {
+    uint64_t sum = 0;
+    for (size_t i = 0; i < n; i++) {
+        const size_t v = orc_ng_get(ng, hashes[i]);
+        if (present) present[i] = (uint8_t)v;
+        sum += v;
+    }
+    return sum;
+}
 /* Nodegraph::update, nodegraph.rs:63-91 (occupied_bins deliberately not updated there).
  * Returns -1 where the reference would panic (a set bit of `other` beyond self's table). */
 int orc_ng_update(OrcNodegraph *ng, const OrcNodegraph *other) {
@@ -931,31 +951,83 @@ double orc_node_containment(const OrcNodegraph *ng, const OrcMinHash *query) {
 /* SBT::find, sbt.rs:147-175, with search_minhashes (mode 0) / search_minhashes_containment (mode 1),
  * search.rs:3-9.  Nodes and leaves are given by tree position; hits_pos receives the positions of the
  * matching leaves in the order the depth-first walk meets them (children are pushed 0..d-1 and popped
- * from the back, so the LAST child is visited first). */
-size_t orc_sbt_find(uint32_t d, const uint64_t *node_pos, OrcNodegraph *const *nodes, const uint64_t *min_n_below,
-                    size_t n_nodes, const uint64_t *leaf_pos, OrcMinHash *const *leaves, size_t n_leaves,
-                    const OrcMinHash *query, int mode, double threshold, uint64_t *hits_pos) {
+ * from the back, so the LAST child is visited first).
+ * orc_sbt_new indexes a tree once for many queries (orc_sbt_query); it copies the position and pointer arrays
+ * but borrows the Nodegraphs and sketches, which must outlive it.  A position listed twice resolves to its
+ * first entry, as a map built by inserting the entries in order and keeping the first. */
+typedef struct { uint64_t pos; size_t idx; } PosIdx;
+typedef struct OrcSbt {
+    uint32_t d;
+    size_t n_nodes, n_leaves;
+    PosIdx *node_at, *leaf_at; /* sorted by (position, index) */
+    OrcNodegraph **nodes;
+    uint64_t *min_n_below;
+    OrcMinHash **leaves;
+} OrcSbt;
+static int pos_idx_cmp(const void *a, const void *b) {
+    const PosIdx *x = (const PosIdx *)a, *y = (const PosIdx *)b;
+    if (x->pos != y->pos) return x->pos < y->pos ? -1 : 1;
+    return x->idx < y->idx ? -1 : x->idx > y->idx;
+}
+static PosIdx *pos_index(const uint64_t *pos, size_t n) {
+    PosIdx *a = (PosIdx *)malloc((n ? n : 1) * sizeof(PosIdx));
+    for (size_t i = 0; i < n; i++) { a[i].pos = pos[i]; a[i].idx = i; }
+    qsort(a, n, sizeof(PosIdx), pos_idx_cmp);
+    return a;
+}
+/* index of the first entry at `pos`, n when there is none */
+static size_t pos_lookup(const PosIdx *a, size_t n, uint64_t pos) {
+    size_t lo = 0, hi = n;
+    while (lo < hi) {
+        const size_t mid = lo + (hi - lo) / 2;
+        if (a[mid].pos < pos) lo = mid + 1; else hi = mid;
+    }
+    return (lo < n && a[lo].pos == pos) ? a[lo].idx : n;
+}
+static void *copy_array(const void *p, size_t n, size_t size) {
+    void *q = malloc((n ? n : 1) * size);
+    if (n) memcpy(q, p, n * size);
+    return q;
+}
+OrcSbt *orc_sbt_new(uint32_t d, const uint64_t *node_pos, OrcNodegraph *const *nodes, const uint64_t *min_n_below,
+                    size_t n_nodes, const uint64_t *leaf_pos, OrcMinHash *const *leaves, size_t n_leaves) {
+    OrcSbt *t = (OrcSbt *)calloc(1, sizeof *t);
+    t->d = d;
+    t->n_nodes = n_nodes;
+    t->n_leaves = n_leaves;
+    t->node_at = pos_index(node_pos, n_nodes);
+    t->leaf_at = pos_index(leaf_pos, n_leaves);
+    t->nodes = (OrcNodegraph **)copy_array(nodes, n_nodes, sizeof *nodes);
+    t->min_n_below = (uint64_t *)copy_array(min_n_below, n_nodes, sizeof *min_n_below);
+    t->leaves = (OrcMinHash **)copy_array(leaves, n_leaves, sizeof *leaves);
+    return t;
+}
+void orc_sbt_free(OrcSbt *t) {
+    if (!t) return;
+    free(t->node_at); free(t->leaf_at); free(t->nodes); free(t->min_n_below); free(t->leaves); free(t);
+}
+size_t orc_sbt_query(const OrcSbt *t, const OrcMinHash *query, int mode, double threshold, uint64_t *hits_pos) {
     size_t n_hits = 0, cap = 64, top = 0;
     uint64_t *stack = (uint64_t *)malloc(cap * sizeof(uint64_t));
     stack[top++] = 0;
     while (top) {
         const uint64_t pos = stack[--top];
         /* positions are unique in a d-ary heap layout, so the reference's `visited` set never fires */
-        size_t ni = n_nodes, li = n_leaves;
-        for (size_t i = 0; i < n_nodes; i++) if (node_pos[i] == pos) { ni = i; break; }
-        if (ni < n_nodes) {
-            const double v = mode ? orc_node_containment(nodes[ni], query) : orc_node_similarity(nodes[ni], min_n_below[ni], query);
+        const size_t ni = pos_lookup(t->node_at, t->n_nodes, pos);
+        if (ni < t->n_nodes) {
+            const double v = mode ? orc_node_containment(t->nodes[ni], query)
+                                  : orc_node_similarity(t->nodes[ni], t->min_n_below[ni], query);
             if (v > threshold) {
-                for (uint32_t c = 0; c < d; c++) {
+                for (uint32_t c = 0; c < t->d; c++) {
                     if (top == cap) { cap *= 2; stack = (uint64_t *)realloc(stack, cap * sizeof(uint64_t)); }
-                    stack[top++] = (uint64_t)d * pos + c + 1;
+                    stack[top++] = (uint64_t)t->d * pos + c + 1;
                 }
             }
             continue;
         }
-        for (size_t i = 0; i < n_leaves; i++) if (leaf_pos[i] == pos) { li = i; break; }
-        if (li < n_leaves) {
-            const double v = mode ? orc_leaf_containment(leaves[li], query) : orc_leaf_similarity(leaves[li], query);
+        const size_t li = pos_lookup(t->leaf_at, t->n_leaves, pos);
+        if (li < t->n_leaves) {
+            const double v = mode ? orc_leaf_containment(t->leaves[li], query) : orc_leaf_similarity(t->leaves[li], query);
             if (v > threshold) hits_pos[n_hits++] = pos;
         }
     }

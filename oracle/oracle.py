@@ -74,6 +74,8 @@ def lib():
             "orc_ng_free": (None, [vp]),
             "orc_ng_count": (i, [vp, u64]),
             "orc_ng_get": (sz, [vp, u64]),
+            "orc_ng_count_many": (u64, [vp, vp, sz, vp]),
+            "orc_ng_get_many": (u64, [vp, vp, sz, vp]),
             "orc_ng_update": (i, [vp, vp]),
             "orc_ng_save": (sz, [vp, C.c_char_p, sz]),
             "orc_ng_load": (vp, [C.c_char_p, sz]),
@@ -82,13 +84,15 @@ def lib():
             "orc_ng_ksize": (sz, [vp]),
             "orc_ng_occupied_bins": (sz, [vp]),
             "orc_ng_unique_kmers": (sz, [vp]),
+            "orc_ng_blocks": (C.POINTER(u32), [vp, sz]),
             "orc_ng_similarity": (C.c_double, [vp, vp]),
             "orc_ng_containment": (C.c_double, [vp, vp]),
             "orc_ng_matches": (u64, [vp, vp]),
             "orc_node_similarity": (C.c_double, [vp, u64, vp]),
             "orc_node_containment": (C.c_double, [vp, vp]),
-            "orc_sbt_find": (sz, [u32, C.POINTER(u64), C.POINTER(vp), C.POINTER(u64), sz, C.POINTER(u64), C.POINTER(vp), sz,
-                                  vp, i, C.c_double, C.POINTER(u64)]),
+            "orc_sbt_new": (vp, [u32, vp, vp, vp, sz, vp, vp, sz]),
+            "orc_sbt_free": (None, [vp]),
+            "orc_sbt_query": (sz, [vp, vp, i, C.c_double, vp]),
         }
         for name, (res, args) in sig.items():
             f = getattr(L, name)
@@ -357,6 +361,20 @@ class Nodegraph:
     def get(self, h):
         return self._L.orc_ng_get(self._p, h)
 
+    def count_many(self, hashes):
+        """(number of new k-mers, count(h) for each hash in batch order as a bool array)"""
+        h = np.ascontiguousarray(hashes, dtype=np.uint64)
+        flags = np.zeros(h.size, dtype=np.uint8)
+        n = self._L.orc_ng_count_many(self._p, h.ctypes.data, h.size, flags.ctypes.data)
+        return n, flags.astype(bool)
+
+    def get_many(self, hashes):
+        """(sum of get(h), get(h) for each hash as a uint8 array)"""
+        h = np.ascontiguousarray(hashes, dtype=np.uint64)
+        flags = np.zeros(h.size, dtype=np.uint8)
+        n = self._L.orc_ng_get_many(self._p, h.ctypes.data, h.size, flags.ctypes.data)
+        return n, flags
+
     def update(self, other):
         if self._L.orc_ng_update(self._p, other._p):
             raise SourmashError(1, "FixedBitSet::put out of bounds")
@@ -372,6 +390,10 @@ class Nodegraph:
 
     def unique_kmers(self):
         return self._L.orc_ng_unique_kmers(self._p)
+
+    def bit(self, t, i):
+        """bit i of table t"""
+        return (self._L.orc_ng_blocks(self._p, t)[i >> 5] >> (i & 31)) & 1
 
     def similarity(self, other):
         return self._L.orc_ng_similarity(self._p, other._p)
@@ -391,17 +413,37 @@ def node_containment(ng, query):  # sbt.rs:256-277
     return lib().orc_node_containment(ng._p, query._p)
 
 
+class SbtOracle:
+    """An SBT indexed once for many SBT::find walks (sbt.rs:147-175).  The tree is given by position as lists, so
+    that a position may be listed twice (its first entry wins): node_positions[i] holds Nodegraph nodes[i] with
+    min_n_below[i], leaf_positions[i] holds KmerMinHash leaves[i]."""
+
+    def __init__(self, d, node_positions, nodes, min_n_below, leaf_positions, leaves):
+        self._L = lib()
+        self._keep = (list(nodes), list(leaves))  # the C index borrows them
+        self.n_leaves = len(leaves)
+        npos = np.ascontiguousarray(node_positions, dtype=np.uint64)
+        mnb = np.ascontiguousarray(min_n_below, dtype=np.uint64)
+        lpos = np.ascontiguousarray(leaf_positions, dtype=np.uint64)
+        assert npos.size == mnb.size == len(nodes) and lpos.size == len(leaves)
+        self._p = self._L.orc_sbt_new(d, npos.ctypes.data, C.cast(_ptr_array(nodes), C.c_void_p), mnb.ctypes.data, npos.size,
+                                      lpos.ctypes.data, C.cast(_ptr_array(leaves), C.c_void_p), lpos.size)
+
+    def __del__(self):
+        if getattr(self, "_p", None):
+            self._L.orc_sbt_free(self._p)
+            self._p = None
+
+    def find(self, query, mode, threshold):
+        """positions of the matching leaves in visit order; mode 'similarity' | 'containment'"""
+        hits = np.zeros(max(1, self.n_leaves), dtype=np.uint64)
+        n = self._L.orc_sbt_query(self._p, query._p, 1 if mode == "containment" else 0, threshold, hits.ctypes.data)
+        return [int(x) for x in hits[:n]]
+
+
 def sbt_find(d, nodes, leaves, query, mode, threshold):
     """SBT::find (sbt.rs:147-175).  nodes: {position: (Nodegraph, min_n_below)}, leaves: {position: KmerMinHash};
     returns the positions of the matching leaves in visit order."""
-    npos = sorted(nodes)
-    lpos = sorted(leaves)
-    a_np = (C.c_uint64 * max(1, len(npos)))(*npos)
-    a_ng = (C.c_void_p * max(1, len(npos)))(*[nodes[p][0]._p for p in npos])
-    a_mb = (C.c_uint64 * max(1, len(npos)))(*[nodes[p][1] for p in npos])
-    a_lp = (C.c_uint64 * max(1, len(lpos)))(*lpos)
-    a_lm = (C.c_void_p * max(1, len(lpos)))(*[leaves[p]._p for p in lpos])
-    hits = (C.c_uint64 * max(1, len(lpos)))()
-    n = lib().orc_sbt_find(d, a_np, a_ng, a_mb, len(npos), a_lp, a_lm, len(lpos), query._p,
-                           1 if mode == "containment" else 0, threshold, hits)
-    return [hits[i] for i in range(n)]
+    npos, lpos = sorted(nodes), sorted(leaves)
+    tree = SbtOracle(d, npos, [nodes[p][0] for p in npos], [nodes[p][1] for p in npos], lpos, [leaves[p] for p in lpos])
+    return tree.find(query, mode, threshold)

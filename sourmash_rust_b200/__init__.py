@@ -791,8 +791,12 @@ def sbt_find(d, nodes, leaf_positions, leaves, queries, mode="similarity", thres
     a_lp = np.ascontiguousarray(leaf_positions, dtype=np.uint64)
     nq = len(queries)
     offs = np.zeros(nq + 1, dtype=np.uint64)
-    cap = max(1, nq * max(1, len(leaf_positions)))
-    hits = np.zeros(cap, dtype=np.uint64)
-    _call("smgpu_sbt_find", d, _vp(a_np), C.cast(a_ng, C.c_void_p), _vp(a_mb), len(npos), _vp(a_lp), leaves._p, queries._p,
-          1 if mode == "containment" else 0, threshold, _vp(offs), _vp(hits), cap)
+    args = (d, _vp(a_np), C.cast(a_ng, C.c_void_p), _vp(a_mb), len(npos), _vp(a_lp), leaves._p, queries._p,
+            1 if mode == "containment" else 0, threshold, _vp(offs))
+    total = _call("smgpu_sbt_find", *args, None, 0)  # the total first, then a buffer of that size
+    hits = np.zeros(max(1, total), dtype=np.uint64)
+    if total:
+        n = _call("smgpu_sbt_find", *args, _vp(hits), total)
+        if n != total:
+            raise RuntimeError("smgpu_sbt_find: %d hits on the second call, %d on the first" % (n, total))
     return [[int(x) for x in hits[int(offs[q]):int(offs[q + 1])]] for q in range(nq)]

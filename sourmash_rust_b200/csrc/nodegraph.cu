@@ -242,7 +242,17 @@ size_t Nodegraph::save(uint8_t *out, size_t cap) {
 }
 
 uint64_t Nodegraph::count_many(const uint64_t *hashes, uint64_t n, uint8_t *is_new, bool on_device) {
-    if (n == 0 || tables.empty()) return 0;
+    if (n == 0) return 0;
+    if (tables.empty()) {  // count() sets no bin, so no hash is new
+        if (is_new && on_device) {
+            Context &ctx = Context::get();
+            SM_CUDA(cudaMemsetAsync(is_new, 0, n, ctx.stream));
+            ctx.sync();
+        } else if (is_new) {
+            std::memset(is_new, 0, n);
+        }
+        return 0;
+    }
     if (n >> NG_TABLE_SHIFT) throw_internal("too many hashes in one count_many call");
     Context &ctx = Context::get();
     cudaStream_t st = ctx.stream;

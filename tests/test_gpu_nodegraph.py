@@ -114,7 +114,9 @@ def test_sbt_find_fixture():  # sbt.rs:543-551 (tree) next to :566-588 (the same
 
 
 # ---- randomised parity ------------------------------------------------------------------------------
-@pytest.mark.parametrize("tablesizes", [[10], [31, 32, 33], [64, 96, 8], [997, 1009, 1013, 1019], [1, 2, 3], [40000, 39989], [255] * 7])
+@pytest.mark.parametrize("tablesizes", [[10], [31, 32, 33], [64, 96, 8], [997, 1009, 1013, 1019], [1, 2, 3], [40000, 39989], [255] * 7,
+                                        [1], [2], [32], [63, 64, 65], [1023, 1024, 1025, 4095, 4096, 4097],
+                                        list(range(1, 256))])
 def test_count_get_random(tablesizes):
     r = splitmix64(sum(tablesizes) + len(tablesizes), 4000)
     g, o = smb.Nodegraph(tablesizes, 21), orc.Nodegraph(tablesizes, 21)

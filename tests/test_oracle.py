@@ -290,3 +290,95 @@ def _is_ancestor(a, pos, d):
     while pos:
         pos = (pos - 1) // d
         yield pos == a
+
+
+@pytest.mark.parametrize("tablesizes", [[10], [1, 2, 31, 32, 33], [997, 1009, 1013, 1019], []])
+def test_nodegraph_batch_calls_equal_the_per_hash_loop(tablesizes):
+    from util import splitmix64
+    r = splitmix64(len(tablesizes) + 17, 3000)
+    batch = np.concatenate([r, r[::7], np.array([0, 1, 2**63, 2**64 - 1], dtype=np.uint64)])
+    one, many = orc.Nodegraph(tablesizes, 21), orc.Nodegraph(tablesizes, 21)
+    for part in (batch[:1], batch[1:2000], batch[2000:]):  # the later parts repeat hashes of the earlier ones
+        want = [one.count(int(h)) for h in part]
+        n, flags = many.count_many(part)
+        assert flags.tolist() == want and n == sum(want)
+        assert many.save() == one.save() and many.unique_kmers() == one.unique_kmers()
+    probe = np.concatenate([r[:500], splitmix64(99, 500)])
+    want = [one.get(int(h)) for h in probe]
+    n, flags = many.get_many(probe)
+    assert flags.tolist() == want and n == sum(want)
+    n, flags = many.count_many([])
+    assert n == 0 and flags.size == 0
+
+
+def _walk_by_scan(d, npos, nodes, mnb, lpos, leaves, query, mode, thr):
+    """SBT::find with each position looked up by a scan that stops at the first entry (the oracle's earlier form)."""
+    hits, stack = [], [0]
+    while stack:
+        pos = stack.pop()
+        if pos in npos:
+            i = npos.index(pos)
+            v = orc.node_containment(nodes[i], query) if mode == "containment" else orc.node_similarity(nodes[i], mnb[i], query)
+            if v > thr:
+                stack.extend(d * pos + c + 1 for c in range(d))
+        elif pos in lpos:
+            i = lpos.index(pos)
+            v = leaves[i].containment(query) if mode == "containment" else leaves[i].similarity(query)
+            if v > thr:
+                hits.append(pos)
+    return hits
+
+
+def _random_tree(d, n_leaves, seed):
+    """A heap-layout tree whose internal nodes hold the hashes of the leaves below them, listed in shuffled order."""
+    from util import splitmix64
+    pool = splitmix64(seed, 4000)
+    n_internal = 1
+    while n_internal * (d - 1) + 1 < n_leaves:
+        n_internal += 1
+    lpos = list(range(n_internal, n_internal + n_leaves))
+    leaves = []
+    for j in range(n_leaves):
+        mh = orc.KmerMinHash(0, 31, False, 42, 2**63)
+        mh.add_many(np.concatenate([pool[j * 40:j * 40 + 40], pool[3000 + (j // 3) * 50:3000 + (j // 3) * 50 + 50]]) >> np.uint64(1))
+        leaves.append(mh)
+    npos, nodes, mnb = [], [], []
+    for p in range(n_internal):
+        below = [leaves[i] for i, lp in enumerate(lpos) if any(_is_ancestor(p, lp, d))]
+        ng = orc.Nodegraph([1999, 2003], 31)
+        for mh in below:
+            ng.count_many(mh.mins_np())
+        npos.append(p)
+        nodes.append(ng)
+        mnb.append(min([mh.size() for mh in below] or [1]))
+    order = np.argsort(splitmix64(seed + 1, n_internal))
+    return ([npos[i] for i in order], [nodes[i] for i in order], [mnb[i] for i in order]), (lpos, leaves)
+
+
+def test_sbt_lookup_matches_a_scan():
+    """The binary-search position lookup gives the hits the first-match scan gives: on the v5 fixture, on random
+    trees, and with a position listed twice (the first entry wins)."""
+    d, nodes, ngs, leaves_d, t = _oracle_tree()
+    npos, lpos = sorted(ngs), sorted(leaves_d)
+    cases = [(d, (npos, [ngs[p][0] for p in npos], [ngs[p][1] for p in npos]), (lpos, [leaves_d[p] for p in lpos]))]
+    for dd, nl, seed in ((2, 13, 1), (3, 20, 2), (5, 31, 3)):
+        cases.append((dd,) + _random_tree(dd, nl, seed))
+    # duplicates: the root listed again after a copy that rejects everything, and a leaf listed twice with different sketches
+    dd, (np_, ng_, mb_), (lp_, lv_) = cases[1]
+    empty = orc.Nodegraph([1999, 2003], 31)
+    cases.append((dd, (np_ + [0], ng_ + [empty], mb_ + [1]), (lp_ + [lp_[0]], lv_ + [lv_[-1]])))
+    cases.append((dd, ([0] + np_, [empty] + ng_, [1] + mb_), ([lp_[0]] + lp_, [lv_[-1]] + lv_)))
+    n_hits = 0
+    for dd, (np_, ng_, mb_), (lp_, lv_) in cases:
+        tree = orc.SbtOracle(dd, np_, ng_, mb_, lp_, lv_)
+        for q in lv_[:6] + [orc.KmerMinHash(0, 31, False, 42, 2**63)]:
+            for mode in ("similarity", "containment"):
+                for thr in (0.0, 0.1, 0.5):
+                    got = tree.find(q, mode, thr)
+                    assert got == _walk_by_scan(dd, np_, ng_, mb_, lp_, lv_, q, mode, thr), (dd, mode, thr)
+                    n_hits += len(got)
+    assert n_hits > 100
+    # the first entry of a duplicated position wins: an empty copy of the root listed first prunes every walk
+    dd, (np_, ng_, mb_), (lp_, lv_) = cases[-1]
+    assert orc.SbtOracle(dd, np_, ng_, mb_, lp_, lv_).find(lv_[1], "containment", 0.0) == []
+    assert orc.SbtOracle(dd, np_[1:], ng_[1:], mb_[1:], lp_, lv_).find(lv_[1], "containment", 0.0) != []
