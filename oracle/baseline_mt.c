@@ -72,6 +72,42 @@ void orc_mt_sketch_reads(const uint8_t *buf, size_t nreads, size_t readlen, cons
 }
 
 typedef struct {
+    const uint8_t *buf;
+    const uint64_t *offsets;
+    size_t n_seqs;
+    uint32_t num, ksize;
+    int is_protein, track;
+    uint64_t seed, max_hash;
+    size_t *next; /* shared: the next sequence to take */
+    OrcMinHash **out;
+} each_job;
+
+static void *each_worker(void *arg) {
+    each_job *j = (each_job *)arg;
+    for (;;) {
+        const size_t s = __atomic_fetch_add(j->next, 1, __ATOMIC_RELAXED);
+        if (s >= j->n_seqs) return NULL;
+        OrcMinHash *mh = orc_mh_new(j->num, j->ksize, j->is_protein, j->seed, j->max_hash, j->track);
+        orc_mh_add_sequence(mh, j->buf + j->offsets[s], (size_t)(j->offsets[s + 1] - j->offsets[s]), 1, NULL);
+        j->out[s] = mh;
+    }
+}
+
+/* One fresh sketch per sequence buf[offsets[s]:offsets[s+1]] (KmerMinHash::new + add_sequence(force = true)), the
+ * sequences taken one at a time by nthreads host threads: the reference loop behind a sketch collection
+ * (lib.rs:142-174, 252-305).  out[s] receives sequence s's sketch (caller frees). */
+void orc_mt_sketch_each(const uint8_t *buf, const uint64_t *offsets, size_t n_seqs, uint32_t num, uint32_t ksize,
+                        int is_protein, uint64_t seed, uint64_t max_hash, int track, int nthreads, OrcMinHash **out) {
+    if (nthreads < 1) nthreads = 1;
+    size_t next = 0;
+    pthread_t *th = (pthread_t *)malloc(sizeof(pthread_t) * (size_t)nthreads);
+    each_job job = {buf, offsets, n_seqs, num, ksize, is_protein, track, seed, max_hash, &next, out};
+    for (int t = 0; t < nthreads; t++) pthread_create(&th[t], NULL, each_worker, &job);
+    for (int t = 0; t < nthreads; t++) pthread_join(th[t], NULL);
+    free(th);
+}
+
+typedef struct {
     OrcMinHash *const *rows; OrcMinHash *const *cols;
     size_t i0, i1, nc;
     uint32_t *common, *size;

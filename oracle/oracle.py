@@ -68,6 +68,7 @@ def lib():
             "orc_signature_json": (vp, [C.c_char_p, C.c_char_p, C.POINTER(vp), sz]),
             "orc_free": (None, [vp]),
             "orc_mt_sketch_reads": (None, [C.c_char_p, sz, sz, C.POINTER(u32), i, u32, u64, i, i, C.POINTER(vp)]),
+            "orc_mt_sketch_each": (None, [C.c_char_p, vp, sz, u32, u32, i, u64, u64, i, i, C.POINTER(vp)]),
             "orc_mt_compare_matrix": (None, [C.POINTER(vp), sz, C.POINTER(vp), sz, vp, vp, i]),
             "orc_mt_compare_pairs": (None, [C.POINTER(vp), vp, vp, sz, vp, vp, i]),
             "orc_ng_new": (vp, [C.POINTER(u64), sz, sz]),
@@ -273,6 +274,19 @@ def scaffold_pairs(leaves):
     a, b = (C.c_uint64 * max(1, n))(), (C.c_uint64 * max(1, n))()
     k = lib().orc_scaffold_pairs(_ptr_array(leaves), n, a, b)
     return [(a[i], None if b[i] == 0xFFFFFFFFFFFFFFFF else b[i]) for i in range(k)]
+
+
+def sketch_each(buf: bytes, offsets, num, ksize, is_protein=False, seed=42, max_hash=0, track_abundance=False,
+                nthreads=None):
+    """One fresh sketch per sequence buf[offsets[s]:offsets[s+1]] (new + add_sequence(force=True)), the sequences
+    spread over nthreads host threads (default: every CPU); returns [KmerMinHash] in sequence order."""
+    o = np.ascontiguousarray(offsets, dtype=np.uint64)
+    n = o.size - 1
+    assert n >= 0 and (n == 0 or int(o[-1]) <= len(buf))
+    out = (C.c_void_p * max(1, n))()
+    lib().orc_mt_sketch_each(buf, o.ctypes.data, n, num, ksize, int(is_protein), seed, max_hash, int(track_abundance),
+                             nthreads or os.cpu_count() or 4, out)
+    return [KmerMinHash(num, ksize, is_protein, seed, max_hash, track_abundance, _ptr=out[s]) for s in range(n)]
 
 
 def compare_matrix(rows, cols, nthreads=1):

@@ -197,6 +197,26 @@ def test_scaled_matches_set_semantics():
     assert mh.abunds == [cnt[h] for h in sorted(cnt)]
 
 
+@pytest.mark.parametrize("num, k, prot, mx, abund", [
+    (0, 21, False, MAX_HASH_1000 * 50, True), (40, 31, False, 0, False), (0, 30, True, 2**64 - 1, False),
+    (25, 24, True, 0, True)])
+def test_sketch_each_equals_the_per_sequence_loop(num, k, prot, mx, abund):
+    lens = [0, 5, 20, 21, 30, 31, 900, 4000, 77, 0, 2500]
+    offsets = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
+    a = bytearray(random_dna(int(offsets[-1]), 0x5EED0002))
+    for p in range(3, len(a), 97):   # invalid bytes and lower case: skipped / upper-cased as add_sequence does
+        a[p] = b"Nn-a"[p % 4]
+    buf = bytes(a)
+    for nthreads in (1, 3, 64):
+        got = orc.sketch_each(buf, offsets, num, k, prot, 7, mx, abund, nthreads)
+        assert len(got) == len(lens)
+        for s, g in enumerate(got):
+            o = orc.KmerMinHash(num, k, prot, 7, mx, abund)
+            o.add_sequence(buf[int(offsets[s]):int(offsets[s + 1])], True)
+            assert g.mins == o.mins and g.abunds == o.abunds, (nthreads, s)
+    assert orc.sketch_each(b"", [0], num, k, prot) == []
+
+
 def test_check_compatible_order():  # lib.rs:176-190
     a = orc.KmerMinHash(10, 21)
     for args, code in (((10, 31), 101), ((10, 21, True), 102), ((10, 21, False, 42, 5), 103),
